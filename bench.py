@@ -2,6 +2,7 @@
 """Benchmark of the TriFinger MDP hot path (reward + obs/states + reset), BASELINE.json metric.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c1|c2|c3|c4|c5] [--all-workloads] [--impl reference]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...      (N > 1, one rank per GPU)
 
 A "step" is one pass of the hot path over all envs of the workload: lg_pre_physics (action store,
@@ -10,10 +11,11 @@ six reward terms, termination, counters, episode statistics).  PhysX is replaced
 synthetic simulator states resident in HBM (leibnizgym_b200/synthetic.py).
 
 One JSON line is printed by rank 0:
-  value      env-steps/s over all GPUs, inputs resident in HBM: the K-step region is replayed from CUDA
-             graphs until >= 50 ms of device time is covered, each repeat timed with CUDA events (max over
-             ranks) in steady state; value = K * envs / median region time (`timing` holds p10 / p90,
-             the repeat count and the cold-start figure)
+  value      env-steps/s over all GPUs, inputs resident in HBM: after the warm-up, exactly K steps are
+             replayed from CUDA graphs and timed with CUDA events (max over ranks) in steady state;
+             value = K * envs / region time (`timing` also holds the cold-start figure).  The window is
+             one sample: at small K it is short (K = 20 is ~0.2 ms at c2) and the figure is noisy, ~1 %
+             from run to run; compare builds at K of about 2048 (the default)
   e2e        the same metric through the public API (VecTaskPython.step + get_state) with the
              simulator state and the action in pinned HOST memory and obs/states/reward/dones
              read back to the host every step
@@ -21,6 +23,9 @@ One JSON line is printed by rank 0:
              against the measured HBM copy bandwidth of MEASURED_PEAKS.json
   cpu_baseline  the oracle port of the reference's torch CPU path on the host cores (N = 1 only)
 `--impl reference` times that CPU path alone and prints the same line shape.
+
+The inputs are generated from the workload's seed, so two runs with the same arguments execute the same steps on the
+same data: `--dump-outputs DIR` writes what the last timed step computed, to compare two builds output for output.
 """
 from __future__ import annotations
 
@@ -336,13 +341,17 @@ def pctl(xs, q):
 
 
 class DeviceTimer:
-    """Steady-state timing of a replayed region with CUDA events, max over ranks.
+    """Steady-state timing of replayed graphs with CUDA events, max over ranks.
 
-    One repeat = barrier + synchronize | one untimed lead-in replay | event | the K-step region (+ the statistics
-    all-reduce when sharded) | event | synchronize.  The lead-in keeps the GPU busy while the host enqueues the timed
-    replays, so the events bracket K steps of a running pipeline, not the launch latency of the first graph of an idle
-    stream (that figure is reported separately as `cold_start_ms_per_step`).  Repeats continue until `min_ms` of timed
-    device time is covered; the result is the median region time and p10 / p90."""
+    `steps` times the K steps of the workload once: barrier + synchronize | lead-in replays | event | the K-step region
+    (+ the statistics all-reduce when sharded) | event | synchronize.  The lead-in keeps the GPU busy while the host
+    enqueues the timed replays, so the events bracket K steps of a running pipeline, not the launch latency of the first
+    graph of an idle stream nor a host-side stall; its first replay starts on an idle stream and is reported as the
+    cold-start figure.  Exactly K steps are timed, so the steps a run executes, and with them its outputs, depend on the
+    arguments only, never on how fast the device is.
+
+    `run` times a single graph (one kernel alone) over repeats until `min_ms` of device time is covered; the result is
+    every repeat's time, for the median and p10 / p90."""
 
     def __init__(self, world: int, dev: str):
         self.world, self.dev = world, dev
@@ -373,6 +382,21 @@ class DeviceTimer:
         torch.cuda.synchronize()
         return e0.elapsed_time(e1)
 
+    def steps(self, region, lead_in, lead_in_reps):
+        """Returns (ms of the first lead-in replay, from an idle stream; region ms), each the max over ranks."""
+        c0, c1, e0, e1 = (torch.cuda.Event(enable_timing=True) for _ in range(4))
+        self.barrier()
+        c0.record()
+        lead_in()
+        c1.record()
+        for _ in range(lead_in_reps - 1):
+            lead_in()
+        e0.record()
+        region()
+        e1.record()
+        torch.cuda.synchronize()
+        return self.agree(c0.elapsed_time(c1)), self.agree(e0.elapsed_time(e1))
+
     def run(self, region, lead_in, min_ms: float = 50.0, min_rep: int = 7, max_rep: int = 400):
         est = self.agree(self.once(region, lead_in))
         reps = int(max(min_rep, min(max_rep, math.ceil(min_ms / max(est, 1e-3)))))
@@ -385,9 +409,13 @@ class DeviceTimer:
         return ms
 
 
-def measure_device(args, wl, rank, world, local_rank, sampler=None):
-    """Device-resident throughput of one workload: K-step regions replayed from CUDA graphs over a ring of simulator
-    states larger than L2, plus the two kernels alone.  Returns a dict of measurements (all times max over ranks)."""
+LEAD_IN_STEPS = 4096    # untimed steps right before the timed ones: ~40 ms of device time at 16384 envs
+
+
+def measure_device(args, wl, rank, world, local_rank, sampler=None, dump_dir=None):
+    """Device-resident throughput of one workload: K steps replayed from CUDA graphs over a ring of simulator states
+    larger than L2, plus the two kernels alone.  Returns a dict of measurements (all times max over ranks).
+    `dump_dir`: rank 0 writes what the last timed step computed there (dump_outputs)."""
     import torch.distributed as dist
 
     from leibnizgym_b200.distributed import stats_to_sums
@@ -452,17 +480,26 @@ def measure_device(args, wl, rank, world, local_rank, sampler=None):
         timer.barrier()
         if sampler is not None:
             sampler.start()
-        ms = timer.run(region, lead_in, min_ms=args.min_timed_ms)
-        cold = [timer.once(region) for _ in range(min(len(ms), 15))]
-        cold_ms = timer.agree(statistics.median(cold))
+        # The lead-in is counted in steps, so the steps before the timed ones are fixed too.  With a single replay
+        # (0.2 ms at K = 20) a host-side stall, such as the clock sampler's thread starting, could leave the device idle
+        # inside the timed region; LEAD_IN_STEPS of queued work absorb it.
+        cold_ms, region_ms = timer.steps(region, lead_in, max(1, math.ceil(LEAD_IN_STEPS / C)))
+        if dump_dir is not None and rank == 0:
+            # every graph starts at ring slot 0: the last timed step wrote output slot (steps in the last graph - 1) % R
+            slot = ((rem or C) - 1) % R
+            per_env = {"obs": runner.obs_slots[slot], "reward": env._reward_buf, "dones": env._dones,
+                       "reset": env._reset_buf, "applied_torque": env._applied_torque}
+            if runner.state_slots is not None:
+                per_env["states"] = runner.state_slots[slot]
+            dump_outputs(dump_dir, per_env, {"step_stats": env._step_stats})
         # ---- the two kernels alone, back to back over the same ring (per-kernel roofline) --------------------------
         Ck = R * max(1, 128 // R)
         post_graph = runner.capture(Ck, post_only=True)
         post_graph.replay()
-        post_ms = timer.run(post_graph.replay, post_graph.replay, min_ms=20.0, min_rep=9, max_rep=60)
+        post_ms = timer.run(post_graph.replay, post_graph.replay, min_ms=args.min_timed_ms, min_rep=9, max_rep=60)
         pre_graph = runner.capture(Ck, pre_only=True)
         pre_graph.replay()
-        pre_ms = timer.run(pre_graph.replay, pre_graph.replay, min_ms=10.0, min_rep=9, max_rep=60)
+        pre_ms = timer.run(pre_graph.replay, pre_graph.replay, min_ms=args.min_timed_ms / 2, min_rep=9, max_rep=60)
         # ---- what a plain device copy of the same number of bytes achieves at this size: R distinct source /
         # destination buffers of half the post kernel's algorithmic bytes each (read + write = the same traffic),
         # copied back to back from a graph like the kernels above.  The roofline peak is measured on a 4 GB copy; a
@@ -478,7 +515,7 @@ def measure_device(args, wl, rank, world, local_rank, sampler=None):
             for t in range(Ck):
                 dst[t % R].copy_(src[t % R])
         copy_graph.replay()
-        copy_ms = timer.run(copy_graph.replay, copy_graph.replay, min_ms=10.0, min_rep=9, max_rep=60)
+        copy_ms = timer.run(copy_graph.replay, copy_graph.replay, min_ms=args.min_timed_ms / 2, min_rep=9, max_rep=60)
         del src, dst
         if sampler is not None:
             sampler.stop()
@@ -499,16 +536,37 @@ def measure_device(args, wl, rank, world, local_rank, sampler=None):
                                             "ok": bool(err < 1e-12 and counts_equal), "ranks": world}
             if not out["stats_allreduce_check"]["ok"]:
                 raise RuntimeError(f"all-reduced statistics differ from the gathered per-rank sums: {out}")
-    med = statistics.median(ms)
     out.update(
-        env=env, cfg=cfg, ring=R, ring_mib=ring.nbytes() / 2**20, steps_per_graph=C, repeats=len(ms),
-        region_ms=med, us_per_step=1e3 * med / K, us_p10=1e3 * pctl(ms, 0.1) / K, us_p90=1e3 * pctl(ms, 0.9) / K,
-        cold_us_per_step=1e3 * cold_ms / K,
+        env=env, cfg=cfg, ring=R, ring_mib=ring.nbytes() / 2**20, steps_per_graph=C,
+        region_ms=region_ms, us_per_step=1e3 * region_ms / K, cold_us_per_step=1e3 * cold_ms / C,
         post_us=1e3 * statistics.median(post_ms) / Ck, post_us_p10=1e3 * pctl(post_ms, 0.1) / Ck,
         post_us_p90=1e3 * pctl(post_ms, 0.9) / Ck, pre_us=1e3 * statistics.median(pre_ms) / Ck,
         copy_us=1e3 * statistics.median(copy_ms) / Ck,
-        value=float(K) * N * world / (med * 1e-3))
+        value=float(K) * N * world / (region_ms * 1e-3))
     return out
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, per_env, other):
+    """Writes each device tensor as <out_dir>/<name>.npy: `per_env` ([N, ...], one row per env; booleans as 0 / 1) in
+    float32, `other` in float64.  When the rows of everything would exceed DUMP_BYTES, a fixed seeded sample of envs is
+    kept, the same rows of every array; env_index.npy lists them."""
+    import numpy as np
+    per_env = {k: v.cpu().numpy() for k, v in per_env.items()}
+    other = {k: v.cpu().numpy().astype(np.float64) for k, v in other.items()}
+    n = len(next(iter(per_env.values())))
+    row_bytes = 8 + sum(4 * (a.size // n) for a in per_env.values())        # + env_index (float64)
+    keep = min(n, (DUMP_BYTES - 4096 * (len(per_env) + len(other) + 1)     # .npy headers
+                   - sum(a.nbytes for a in other.values())) // row_bytes)
+    rows = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in per_env.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a[rows].astype(np.float32))
+    np.save(os.path.join(out_dir, "env_index.npy"), rows.astype(np.float64))
+    for name, a in other.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def summarize_workload(wl, m):
@@ -519,10 +577,10 @@ def summarize_workload(wl, m):
     post_gbs = POST_BYTES[asym] * N / (m["post_us"] * 1e-6) / 1e9
     step_bytes = (POST_BYTES[asym] + PRE_BYTES + (wl["reset_p"] + wl.get("goal_p", 0.0) / 3) * RESET_BYTES) * N
     return {"workload": wl["desc"], "envs_per_gpu": N, "value": m["value"], "us_per_step": m["us_per_step"],
-            "us_p10": m["us_p10"], "us_p90": m["us_p90"], "post_us": m["post_us"], "pre_us": m["pre_us"],
+            "post_us": m["post_us"], "pre_us": m["pre_us"],
             "post_frac_of_hbm_peak": post_gbs / peak,
             "whole_step_frac_of_hbm_peak": step_bytes / (m["us_per_step"] * 1e-6) / 1e9 / peak,
-            "repeats": m["repeats"], "ring": m["ring"]}
+            "ring": m["ring"]}
 
 
 def run_gpu(args, wl):
@@ -546,7 +604,7 @@ def run_gpu(args, wl):
     asym = wl["asym"]
     # clocks are sampled on rank 0 only (one NVML thread per box, 20 ms period), while the timed repeats run
     sampler = ClockSampler(physical_gpu_index(local_rank), period_s=0.02) if rank == 0 else None
-    m = measure_device(args, wl, rank, world, local_rank, sampler)
+    m = measure_device(args, wl, rank, world, local_rank, sampler, dump_dir=args.dump_outputs)
     m.pop("env")
     cfg = m.pop("cfg")
     clocks = sampler.summary() if sampler is not None else None
@@ -570,11 +628,10 @@ def run_gpu(args, wl):
         "metric": METRIC, "value": m["value"], "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
         "ms_per_step": m["us_per_step"] * 1e-3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "f32", "data": "synthetic", "config": config,
-        "timing": {"method": "CUDA events around the K-step region replayed from CUDA graphs, after one untimed lead-in "
-                             "replay (steady state); barrier + synchronize around every repeat; per repeat the max over "
-                             "ranks; value = median over repeats",
-                   "repeats": m["repeats"], "steps_per_graph": m["steps_per_graph"], "region_ms_median": m["region_ms"],
-                   "us_per_step_median": m["us_per_step"], "us_per_step_p10": m["us_p10"], "us_per_step_p90": m["us_p90"],
+        "timing": {"method": f"CUDA events around the K steps, replayed from CUDA graphs once, after an untimed lead-in "
+                             f"of >= {LEAD_IN_STEPS} steps (steady state); the max over ranks; value = K steps / region "
+                             f"time; cold start = the first lead-in replay (steps_per_graph steps), from an idle stream",
+                   "steps_per_graph": m["steps_per_graph"], "region_ms": m["region_ms"], "us_per_step": m["us_per_step"],
                    "cold_start_us_per_step": m["cold_us_per_step"],
                    "statistics_allreduce_in_region": world > 1,
                    "pre_launch": "stream order (lg_pre_physics)" if args.no_chain else
@@ -715,7 +772,13 @@ def main():
     ap.add_argument("--ring", type=int, default=0, help="distinct simulator states in HBM (0: sized to several times L2)")
     ap.add_argument("--all-workloads", action="store_true",
                     help="also measure one line per BASELINE.json config (c1, c1sym, c2, c3ref, c4, c5) into `workloads`")
-    ap.add_argument("--min-timed-ms", type=float, default=50.0, help="repeat the K-step region until this much device time is covered")
+    ap.add_argument("--min-timed-ms", type=float, default=20.0,
+                    help="device time the kernel-alone roofline timings repeat for: the post-physics kernel this long, "
+                         "the pre-physics kernel and the device copy half of it (the K timed steps are not repeated)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0's envs: obs, states, reward, dones, reset, "
+                         "applied_torque, step_stats) as DIR/<name>.npy, float32 / float64; at most 64 MB, a seeded "
+                         "sample of envs (env_index.npy) when larger")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-chain", action="store_true",
                     help="launch the pre-physics pass in stream order (lg_pre_physics) instead of chained to the preceding "
@@ -733,6 +796,8 @@ def main():
         wl["envs"] = args.envs
         wl["desc"] += f" [envs/GPU overridden to {args.envs}]"
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the outputs of the B200 path; it does not apply to --impl reference")
         run_reference(args, wl)
         return
     if not torch.cuda.is_available():

@@ -15,8 +15,8 @@ import json
 try:
     d = json.loads(open("gpurun_out/ab_${v}_$wl.json").read().strip().splitlines()[-1])
     r, t = d["roofline"], d["timing"]
-    print("[$v] $wl step %.2f us (p10 %.2f p90 %.2f, cold %.2f) post %.2f pre %.2f frac %.3f whole %.3f copy %.2f" % (
-        t["us_per_step_median"], t["us_per_step_p10"], t["us_per_step_p90"], t["cold_start_us_per_step"], r["launch_us"], r["pre_us"], r["frac"], r["whole_step_frac"], r["device_copy_same_bytes_us"]))
+    print("[$v] $wl step %.2f us (cold %.2f) post %.2f pre %.2f frac %.3f whole %.3f copy %.2f" % (
+        t["us_per_step"], t["cold_start_us_per_step"], r["launch_us"], r["pre_us"], r["frac"], r["whole_step_frac"], r["device_copy_same_bytes_us"]))
 except Exception as ex:
     print("[$v] $wl FAILED", ex)
 PY

@@ -1,162 +1,45 @@
-"""Property-style pin of the oracle's building blocks against the UNMODIFIED reference functions, on random and
+"""Property-style pin of the oracle's building blocks against the reference functions' outputs, on random and
 adversarial inputs — a wider net than the 12 stored scenarios.
 
-Runs only where the reference tree is mounted (the build container: /root/reference or $LEIBNIZ_REFERENCE_ROOT); it is
-skipped on the GPU box, where the committed fixtures of tests/golden/ play that role.  CPU only; the reference's
-functions are called both through TorchScript (its real path) and bit-compared with the oracle's eager restatement.
+The inputs are rebuilt from fixed seeds by tests/golden/reference_functions.py; the outputs they are compared with bit
+for bit are stored in tests/golden/functions/reference_functions.npz (how it was recorded, and how to record it again
+from the reference's own functions, is described there).  CPU only.
 """
-import importlib.util
-import math
 import os
 import sys
-import types
 
 import numpy as np
 import pytest
-import torch
 
-REF = os.environ.get("LEIBNIZ_REFERENCE_ROOT", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "leibnizgym")),
-                                reason="reference tree not mounted (fixtures in tests/golden cover the GPU box)")
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+import reference_functions as rf  # noqa: E402
 
 
 @pytest.fixture(scope="module")
-def ref():
-    """The reference's pure modules, imported from where they lie (nothing is copied)."""
-    saved = {k: sys.modules.get(k) for k in ("termcolor", "leibnizgym", "leibnizgym.utils", "leibnizgym.utils.torch_utils",
-                                             "leibnizgym.utils.mdp", "leibnizgym.utils.message")}
-    tc = types.ModuleType("termcolor")
-    tc.colored = lambda s, *a, **k: s
-    sys.modules["termcolor"] = tc
-
-    def load(name, rel):
-        spec = importlib.util.spec_from_file_location(name, os.path.join(REF, rel))
-        mod = importlib.util.module_from_spec(spec)
-        sys.modules[name] = mod
-        spec.loader.exec_module(mod)
-        return mod
-
-    pkg = types.ModuleType("leibnizgym"); pkg.__path__ = []          # noqa: E702
-    utils = types.ModuleType("leibnizgym.utils"); utils.__path__ = []  # noqa: E702
-    sys.modules["leibnizgym"], sys.modules["leibnizgym.utils"] = pkg, utils
-    tu = load("leibnizgym.utils.torch_utils", "leibnizgym/utils/torch_utils.py")
-    load("leibnizgym.utils.mdp", "leibnizgym/utils/mdp.py")
-    rw = load("_ref_rewards", "leibnizgym/envs/trifinger/rewards.py")
-    sm = load("_ref_sample", "leibnizgym/envs/trifinger/sample.py")
-    yield types.SimpleNamespace(tu=tu, rw=rw, sm=sm)
-    for k, v in saved.items():
-        if v is None:
-            sys.modules.pop(k, None)
-        else:
-            sys.modules[k] = v
+def stored():
+    with np.load(rf.PATH) as z:
+        return {k: z[k] for k in z.files}
 
 
-def _same(a, b):
-    a, b = a.detach().numpy(), b.detach().numpy()
-    return bool(np.all((a == b) | (np.isnan(a) & np.isnan(b))))
+def _check(stored, group, got):
+    want = sorted(k for k in stored if k.startswith(group + "/"))
+    assert want == sorted(f"{group}/{k}" for k in got), group
+    for k, v in got.items():
+        assert rf.same(v.detach().numpy(), stored[f"{group}/{k}"]), (group, k)
 
 
-def _quats(g, n, unit=True):
-    q = torch.randn(n, 4, generator=g)
-    return q / q.norm(dim=1, keepdim=True) if unit else q
+def test_primitives_bit_exact(stored):
+    """scale / unscale / saturate, quaternion product, conjugate, angle, from-Euler and the lgsk kernel."""
+    _check(stored, "primitives", rf.primitives())
 
 
-def _poses(g, n):
-    p = torch.zeros(n, 13)
-    p[:, 0:3] = torch.rand(n, 3, generator=g) * 0.6 - 0.3
-    p[:, 3:7] = _quats(g, n)
-    p[:, 7:13] = torch.randn(n, 6, generator=g) * 0.1
-    return p
+@pytest.mark.parametrize("seed", rf.REWARD_SEEDS)
+def test_reward_terms_bit_exact_over_random_schedules(stored, seed):
+    """The six reward terms against the reference's scripted modules (trifinger_env.py:350): random weights, scales and
+    schedule windows, env-step counts on, inside and outside the windows."""
+    _check(stored, f"reward{seed}", rf.reward_terms(seed))
 
 
-def test_primitives_bit_exact(ref):
-    import oracle.trifinger_oracle as o
-    g = torch.Generator().manual_seed(1)
-    N = 50_000
-    x = torch.randn(N, 9, generator=g) * 3
-    x[:5] = torch.tensor([0.0, -0.0, 1e-42, 3.4e38, -3.4e38, float("inf"), 1.0, -1.0, 0.5])[None]
-    lo, hi = -torch.rand(9, generator=g) - 0.1, torch.rand(9, generator=g) + 0.1
-    for mine, theirs in ((o.scale_transform, ref.tu.scale_transform), (o.unscale_transform, ref.tu.unscale_transform),
-                         (o.saturate, ref.tu.saturate)):
-        assert _same(mine(x, lo, hi), theirs(x, lo, hi)), theirs
-    a, b = _quats(g, N), _quats(g, N)
-    b[:100] = a[:100]                     # identical
-    b[100:200] = -a[100:200]              # antipodal
-    a[200:300] = _quats(g, 100, unit=False) * 3   # non-unit: |v| > 1 -> clamp
-    a[300] = 0.0                           # zero quaternion
-    assert _same(o.quat_mul(a, b), ref.tu.quat_mul(a, b))
-    assert _same(o.quat_conjugate(a), ref.tu.quat_conjugate(a))
-    assert _same(o.quat_diff_rad(a, b), ref.tu.quat_diff_rad(a, b))
-    r, p, y = (torch.rand(N, generator=g) * 2 * math.pi for _ in range(3))
-    assert _same(o.quat_from_euler_xyz(r, p, y), ref.tu.quaternion_from_euler_xyz(r, p, y))
-    d = torch.cat([torch.rand(N, generator=g) * 2.5, torch.tensor([0.0, 1.78, 1.8, 5.0, 1e-30])])
-    for scale in (50.0, 30.0, 3.0):
-        assert _same(o.lgsk(d, scale), ref.rw.lgsk_kernel(d, scale))
-
-
-@pytest.mark.parametrize("seed", [0, 1, 2])
-def test_reward_terms_bit_exact_over_random_schedules(ref, seed):
-    """The six reward modules (scripted, as trifinger_env.py:350 does) against the oracle's terms: random weights,
-    scales and schedule windows, env-step counts on, inside and outside the windows."""
-    import oracle.trifinger_oracle as o
-    g = torch.Generator().manual_seed(100 + seed)
-    rs = np.random.RandomState(seed)
-    N, dt = 4096, 0.02
-    obj, obj_prev, goal = _poses(g, N), _poses(g, N), _poses(g, N)[:, :7].contiguous()
-    tips = torch.stack([_poses(g, N) for _ in range(3)], dim=1)
-    tips_prev = torch.stack([_poses(g, N) for _ in range(3)], dim=1)
-    obj[:64, 0:7] = goal[:64]                                  # on the goal: d = 0, theta = 0
-    tips[64:96, :, 0:3] = obj[64:96, None, 0:3]                # fingertips in the cube centre
-    start, end = float(rs.randint(0, 1000)), float(rs.randint(1000, 5000))
-    cfg = {
-        "finger_reach_object_rate": {"activate": True, "weight": float(-rs.randint(1, 900)), "norm_p": 2,
-                                     "thresh_sched_start": start, "thresh_sched_end": end},
-        "finger_move_penalty": {"activate": True, "weight": -float(rs.rand())},
-        "object_dist": {"activate": True, "weight": float(rs.randint(1, 3000)),
-                        "thresh_sched_start": start, "thresh_sched_end": end},
-        "object_rot": {"activate": True, "weight": float(rs.randint(1, 3000)), "scale": float(1 + 4 * rs.rand()),
-                       "epsilon": 0.01, "thresh_sched_start": start, "thresh_sched_end": end},
-        "object_rot_delta": {"activate": True, "weight": float(-rs.randint(1, 500)),
-                             "linear_schedule_start": start, "linear_schedule_end": end},
-        "object_move": {"activate": True, "weight": float(-rs.randint(1, 900))},
-    }
-    classes = {"finger_reach_object_rate": ref.rw.FingerReachObjectRatePenalty, "finger_move_penalty": ref.rw.FingertipMovementPenalty,
-               "object_dist": ref.rw.ObjectDistanceReward, "object_rot": ref.rw.ObjectRotationReward,
-               "object_rot_delta": ref.rw.ObjectRotationDeltaReward, "object_move": ref.rw.ObjectMoveReward}
-    mods = {k: torch.jit.script(classes[k](name=k, **dict(v))) for k, v in cfg.items()}
-    P = o.reward_term_params(cfg)
-    for T in (0.0, start, start + 1.0, 0.5 * (start + end), end, end + 1.0, 1e9):
-        pairs = [
-            (o.finger_reach_object_rate(P["finger_reach_object_rate"], T, tips, tips_prev, obj, obj_prev),
-             mods["finger_reach_object_rate"].compute(T, tips, tips_prev, obj, obj_prev)),
-            (o.finger_move_penalty(P["finger_move_penalty"], dt, tips, tips_prev),
-             mods["finger_move_penalty"].compute(dt, tips, tips_prev)),
-            (o.object_dist(P["object_dist"], dt, T, obj, goal), mods["object_dist"].compute(dt, T, obj, goal)),
-            (o.object_rot(P["object_rot"], dt, T, obj, goal), mods["object_rot"].compute(dt, T, obj, goal)),
-            (o.object_rot_delta(P["object_rot_delta"], dt, T, obj, obj_prev, goal),
-             mods["object_rot_delta"].compute(dt, T, obj, obj_prev, goal)),
-            (o.object_move(P["object_move"], obj, obj_prev, goal), mods["object_move"].compute(obj, obj_prev, goal)),
-        ]
-        for i, (mine, theirs) in enumerate(pairs):
-            assert _same(mine, theirs), (seed, T, i)
-
-
-def test_samplers_consume_the_generator_like_the_reference(ref):
+def test_samplers_consume_the_generator_like_the_reference(stored):
     """Same seed, same call order -> same samples: the oracle's samplers draw what sample.py draws (CPU generator)."""
-    import oracle.trifinger_oracle as o
-    k = 1000
-    torch.manual_seed(123)
-    rx, ry = ref.sm.random_xy(k, 0.15, "cpu")
-    rz = ref.sm.random_z(k, 0.03, 0.2, "cpu")
-    rq = ref.sm.random_orientation(k, "cpu")
-    rw = ref.sm.random_angular_vel(k, "cpu", 0.5)
-    ryaw = ref.sm.random_yaw_orientation(k, "cpu")
-    torch.manual_seed(123)
-    d = o.Draws()                        # draws from torch global generator, in the reference order
-    x, y = o.random_xy(d, k, 0.15, (0, 1))
-    z = o.random_z(d, k, 0.03, 0.2, 2)
-    q = o.random_orientation(d, k)
-    w = o.random_angular_vel(d, k, 0.5)
-    yaw = o.random_yaw_orientation(d, k, 3)
-    for mine, theirs in ((x, rx), (y, ry), (z, rz), (q, rq), (w, rw), (yaw, ryaw)):
-        assert _same(mine, theirs)
+    _check(stored, "samplers", rf.samplers())
