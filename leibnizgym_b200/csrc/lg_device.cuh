@@ -137,9 +137,24 @@ __device__ __forceinline__ float unscale_transform(float x, float lo, float hi) 
   const float centre = (lo + hi) * 0.5f;
   return (x * (hi - lo)) * 0.5f + centre;
 }
-__device__ __forceinline__ float saturate(float x, float lo, float hi) {  // torch_utils.py:60-75
-  return fmaxf(fminf(x, hi), lo);
+// torch.min / torch.max / torch.clamp propagate NaN; fminf / fmaxf would return the other operand and turn a diverged
+// value into a legal-looking bound.  min.NaN / max.NaN compile to one FMNMX.NAN each (fminf / fmaxf: one FMNMX) and
+// give the same bits for every non-NaN input.
+__device__ __forceinline__ float min_nan(float a, float b) {
+  float r;
+  asm("min.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+  return r;
 }
+__device__ __forceinline__ float max_nan(float a, float b) {
+  float r;
+  asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+  return r;
+}
+__device__ __forceinline__ float saturate(float x, float lo, float hi) {  // torch_utils.py:60-75: max(min(x, hi), lo)
+  return max_nan(min_nan(x, hi), lo);
+}
+// torch.clamp(x, lo, hi) (wrappers/vec_task.py:147, :162, :167)
+__device__ __forceinline__ float clamp_nan(float x, float lo, float hi) { return min_nan(max_nan(x, lo), hi); }
 
 // 1 / (e^{s x} + 2 + e^{-s x}) (envs/trifinger/rewards.py:20-34); generalised eps for the extension
 __device__ __forceinline__ float lgsk(float x, float scale, float eps = 2.0f) {

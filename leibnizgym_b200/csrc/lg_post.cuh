@@ -696,13 +696,13 @@ post_physics_kernel(const __grid_constant__ LgParams P, const __grid_constant__ 
       auto emit_one = [&](int k, float sv, float ov) {
         if (ASYM) {
           __stcs(st + k * L::STATE, sv);
-          const float svc = CLIP ? fminf(fmaxf(sv, -clip), clip) : sv;
+          const float svc = CLIP ? clamp_nan(sv, -clip, clip) : sv;
           if (CLIP) __stcs(stc + k * L::STATE, svc);
           if (EXT && stb) __stcs(stb + k * L::STATE, to_bf16(svc));
         }
         if (to_obs) {
           __stcs(ob + k * L::OBS, ov);
-          const float ovc = CLIP ? fminf(fmaxf(ov, -clip), clip) : ov;
+          const float ovc = CLIP ? clamp_nan(ov, -clip, clip) : ov;
           if (CLIP) __stcs(obc + k * L::OBS, ovc);
           if (EXT && obb) __stcs(obb + k * L::OBS, to_bf16(ovc));
         }

@@ -442,7 +442,7 @@ pre_physics_kernel(const __grid_constant__ PreHot H, const __grid_constant__ LgP
       if (P.clip_input_actions) {   // the wrapper's clamp (wrappers/vec_task.py:162)
         const float clip = P.clip_actions;
 #pragma unroll
-        for (int c = 0; c < A; ++c) act[c] = fminf(fmaxf(act[c], -clip), clip);
+        for (int c = 0; c < A; ++c) act[c] = clamp_nan(act[c], -clip, clip);
       }
       if (zero_row) {               // the row is zeroed after the store (envs/env_base.py:369, trifinger_env.py:387)
 #pragma unroll

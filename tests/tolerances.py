@@ -51,12 +51,16 @@ def compare(key, got, expected, extra_atol=None):
         ok = np.array_equal(got.astype(np.int64), expected.astype(np.int64))
         return ok, "" if ok else f"{int((got.astype(np.int64) != expected.astype(np.int64)).sum())} entries differ"
     g, x = got.astype(np.float64), expected.astype(np.float64)
-    err = np.abs(g - x)
+    with np.errstate(invalid="ignore"):
+        err = np.abs(g - x)   # inf - inf is NaN
     bound = ATOL[key] + RTOL * np.abs(x)
     if extra_atol is not None:
         bound = bound + np.asarray(extra_atol, dtype=np.float64)
-    bad = ~((err <= bound) | (np.isnan(g) & np.isnan(x)))
+    # The relative bound applies to finite expectations only (RTOL * inf would accept anything).  Equal values agree
+    # (an infinity equals itself; -0.0 == +0.0, which the fast division's -0 -> +0 needs) and NaN agrees with NaN.
+    close = np.isfinite(x) & (err <= bound)
+    bad = ~(close | (g == x) | (np.isnan(g) & np.isnan(x)))
     if bad.any():
-        i = np.unravel_index(np.argmax(np.where(bad, err, 0)), err.shape)
+        i = np.unravel_index(np.argmax(np.where(bad, np.nan_to_num(err, nan=np.inf), -1.0)), err.shape)
         return False, f"{int(bad.sum())} entries off; worst at {i}: got {g[i]!r} expected {x[i]!r} err {err[i]:.3e}"
-    return True, f"max abs err {err.max() if err.size else 0:.3e}"
+    return True, f"max abs err {np.where(close, err, 0).max() if err.size else 0:.3e}"
