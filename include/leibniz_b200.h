@@ -57,6 +57,11 @@ enum LgTerm {
 
 enum LgCommandMode { LG_CMD_POSITION = 0, LG_CMD_TORQUE = 1, LG_CMD_POSITION_IMPEDANCE = 2 };
 enum LgResetKind { LG_RESET_NONE = 0, LG_RESET_DEFAULT = 1, LG_RESET_RANDOM = 2 };
+/* Where reset and goal samples come from (LgParams.rng_stream):
+ *   LG_RNG_PHILOX  the library's own Philox stream keyed by (seed, global env id, purpose, epoch): sharding-invariant;
+ *   LG_RNG_TORCH   the elements torch.rand / torch.randn on this CUDA device would return for the reference's own
+ *                  calls (LgTorchRng): a seeded run samples what a seeded reference run samples.  One shard only. */
+enum LgRngStream { LG_RNG_PHILOX = 0, LG_RNG_TORCH = 1 };
 
 /* slots of the statistics vector (sums over the envs of this shard; the reference's
  * `_step_info` means are sum / num_envs — trifinger_env.py:554, :1067-1068, :1076, :1098-1099) */
@@ -140,6 +145,10 @@ typedef struct LgParams {
   float dr_action_sigma;
   float dr_sigma[LG_MAX_STATE_DIM];
   int32_t _pad_tail;
+  int32_t rng_stream;       /* LgRngStream                                                          */
+  int32_t sm_count;         /* LG_RNG_TORCH: the device's multiProcessorCount and                   */
+  int32_t threads_per_sm;   /* maxThreadsPerMultiProcessor, which fix torch's launch grid           */
+  int32_t _pad_tail2;
 } LgParams;
 
 /* Scalar coefficients of the reward terms for ONE value of env_steps_count: the Python-float
@@ -159,6 +168,19 @@ typedef struct LgControl {
   uint32_t scan_readers;  /* direct-prefix variant of lg_pre_physics: tiles that have read their predecessors' flags */
   uint32_t scan_exits;    /* ... and tiles that have finished; the last one re-arms both and advances scan_epoch   */
 } LgControl;
+
+/* State of torch's CUDA Philox generator as LG_RNG_TORCH draws from it (device-resident, one per env).  `seed` and
+ * `offset` are what torch.cuda.manual_seed / Generator.get_offset() hold; every launch that draws advances `offset` as
+ * the reference's calls would.  The rest is workspace of lg_pre_physics (zero-initialise it). */
+typedef struct LgTorchRng {
+  uint64_t seed;
+  uint64_t offset;
+  uint64_t launch_base;     /* offset the current lg_pre_physics launch draws from                  */
+  int32_t launch_counts[2]; /* its reset / goal-reset list lengths                                  */
+  uint32_t acc[2];          /* counting launch: running list lengths (re-armed to 0)                */
+  uint32_t ticket;          /* counting launch: CTAs done (re-armed to 0)                           */
+  uint32_t _pad;
+} LgTorchRng;
 
 /* The simulator-owned tensors (zero-copy views in the reference, trifinger_env.py:602-617). */
 typedef struct LgSimState {
@@ -217,6 +239,7 @@ typedef struct LgBuffers {
      caller does with `env._reset_buf |= mask` between steps (tests, reset-heavy workloads), without a separate pass */
   const uint8_t* force_reset;
   const uint8_t* force_goal_reset;
+  LgTorchRng* torch_rng;    /* P.rng_stream == LG_RNG_TORCH: the generator state (NULL otherwise)  */
 } LgBuffers;
 
 int lg_version(void);
@@ -291,6 +314,14 @@ int lg_reset_envs(const LgParams* P, const LgSimState* S, const LgBuffers* B,
                   const int64_t* ids, int64_t k_host, void* stream);
 int lg_goal_reset_envs(const LgParams* P, const LgSimState* S, const LgBuffers* B,
                        const int64_t* ids, int64_t k_host, void* stream);
+
+/* torch's CUDA uniform / normal stream as a batched primitive: out[0..n) = what torch.rand(n) (normal == 0) or
+ * torch.randn(n) (normal != 0) returns in fp32 on the current device for a generator with this seed and Philox
+ * offset (a multiple of 4).  Advances nothing.  n < 2^31. */
+int lg_torch_philox(uint64_t seed, uint64_t offset, int64_t n, int normal, float* out, void* stream);
+/* Host only: how far such a call advances the generator's offset on a device with `sm_count` SMs of
+ * `threads_per_sm` threads (0 for n == 0). */
+uint64_t lg_torch_philox_advance(int64_t n, int32_t sm_count, int32_t threads_per_sm);
 
 /* _pre_step alone (trifinger_env.py:442-498) on the current _action_buf */
 int lg_pre_step(const LgParams* P, const LgSimState* S, const LgBuffers* B, void* stream);

@@ -27,6 +27,7 @@ TERM_NAMES = ("finger_reach_object_rate", "finger_move_penalty", "object_dist", 
               "object_rot_delta", "object_move", "keypoint")
 CMD_MODES = {"position": 0, "torque": 1, "position_impedance": 2}
 RESET_KINDS = {"none": 0, "default": 1, "random": 2}
+RNG_STREAMS = {"philox": 0, "torch": 1}
 STAT_POSITION_GOAL, STAT_ORIENTATION_GOAL, STAT_SUCCESSES, STAT_REWARD, STAT_RESETS, STAT_DONES = 7, 8, 9, 10, 11, 12
 
 c_float_p = C.POINTER(C.c_float)
@@ -65,12 +66,18 @@ class LgParams(C.Structure):
         ("cube_half_size", C.c_double), ("cube_radius_3d", C.c_double), ("cube_max_height", C.c_double),
         ("max_com_distance", C.c_double),
         ("dr_action_sigma", C.c_float), ("dr_sigma", C.c_float * LG_MAX_STATE_DIM), ("_pad_tail", C.c_int32),
+        ("rng_stream", C.c_int32), ("sm_count", C.c_int32), ("threads_per_sm", C.c_int32), ("_pad_tail2", C.c_int32),
     ]
 
 
 class LgControl(C.Structure):
     _fields_ = [("rng_epoch", C.c_uint64), ("frame_count", C.c_int64), ("scan_ticket", C.c_uint32),
                 ("scan_epoch", C.c_uint32), ("scan_readers", C.c_uint32), ("scan_exits", C.c_uint32)]
+
+
+class LgTorchRng(C.Structure):
+    _fields_ = [("seed", C.c_uint64), ("offset", C.c_uint64), ("launch_base", C.c_uint64),
+                ("launch_counts", C.c_int32 * 2), ("acc", C.c_uint32 * 2), ("ticket", C.c_uint32), ("_pad", C.c_uint32)]
 
 
 class LgSimState(C.Structure):
@@ -85,7 +92,7 @@ class LgBuffers(C.Structure):
         "term_rewards", "step_stats", "reset_ids", "goal_reset_ids", "counts",
         "robot_indices", "reset_root_indices", "goal_root_indices", "scan_status", "control", "reward_coef", "scale_table",
         "inject_reset_u", "inject_reset_n", "inject_goal_u", "inject_goal_n", "obs_bf16", "states_bf16",
-        "force_reset", "force_goal_reset")]
+        "force_reset", "force_goal_reset", "torch_rng")]
 
 
 class LgHostStep(C.Structure):
@@ -125,6 +132,8 @@ SYMBOLS = {
     "lg_upload_sim_state": (C.c_int, [_P, _S, C.POINTER(LgHostStep), _vp]),
     "lg_step_host_pipelined": (C.c_int, [_P, _S, _B, C.POINTER(LgHostStep), C.c_double, C.c_int, _vp, _vp, _vp]),
     "lg_step_host": (C.c_int, [_P, _S, _B, C.POINTER(LgHostStep), C.c_double, _vp]),
+    "lg_torch_philox": (C.c_int, [C.c_uint64, C.c_uint64, _i64, C.c_int, _vp, _vp]),
+    "lg_torch_philox_advance": (C.c_uint64, [_i64, _i32, _i32]),
 }
 
 
@@ -148,7 +157,7 @@ def load() -> C.CDLL:
     for name, (res, args) in SYMBOLS.items():
         fn = getattr(lib, name)  # AttributeError if the .so lacks a declared symbol
         fn.restype, fn.argtypes = res, args
-    for which, struct in enumerate((LgParams, LgSimState, LgBuffers, LgControl, LgRewardTerm, LgHostStep)):
+    for which, struct in enumerate((LgParams, LgSimState, LgBuffers, LgControl, LgRewardTerm, LgHostStep, LgTorchRng)):
         native = lib.lg_struct_size(which)
         if native != C.sizeof(struct):
             raise NativeError(f"ABI mismatch: sizeof({struct.__name__}) is {native} in the library, "

@@ -4,8 +4,8 @@ The reference has no resume path for the environment (SURVEY.md §5; `dump_confi
 envs/env_base.py:295-309, only writes the config).  A run of this build can stop after any step
 and continue bit-identically: the file holds the goal poses and movement, step counters, reset /
 goal-reset / success flags, the one-deep history, the last action / outputs, the per-step
-statistics, and the device control block (RNG epoch of the kernel's Philox stream, frame counter,
-compaction epoch) — plus, for `SyntheticSim`, the simulator tensors and its clock, because the
+statistics, the device control block (RNG epoch of the kernel's Philox stream, frame counter,
+compaction epoch) and the state of the torch CUDA stream (`rng_stream` "torch": seed, offset) — plus, for `SyntheticSim`, the simulator tensors and its clock, because the
 pre-physics pass of the next step reads (and the resets wrote) simulator memory.
 
 Format: one uncompressed `.npz`; `meta` is a JSON string (format version, shard geometry, config),
@@ -30,7 +30,7 @@ _ENV_TENSORS = {
     "goal_pose": "_object_goal_poses_buf", "goal_movement": "_object_goal_movement_buf", "history": "_history",
     "applied_torque": "_applied_torque", "step_stats": "_step_stats", "control": "_control",
     "scan_status": "_scan_status", "counts": "_counts", "reset_ids": "_reset_ids", "goal_reset_ids": "_goal_reset_ids",
-    "reward_coef": "_reward_coef",
+    "reward_coef": "_reward_coef", "torch_rng": "_torch_rng",
 }
 _SIM_TENSORS = ("dof_state", "root_state", "rigid_body", "dof_force", "ft_sensors")
 
@@ -69,6 +69,11 @@ def load_env_state_dict(env, state: Dict[str, object]) -> None:
                       ("state_dim", env.get_state_dim()), ("action_dim", env.get_action_dim())):
         if int(meta[key]) != int(have):
             raise ValueError(f"checkpoint was written for {key}={meta[key]}, this env has {have}")
+    # the two streams are different random sequences (and "torch" carries generator state): never mix them
+    have_stream = env.config.get("rng_stream", "philox")
+    ck_stream = meta.get("config", {}).get("rng_stream", "philox")
+    if ck_stream != have_stream:
+        raise ValueError(f"checkpoint was written with rng_stream={ck_stream!r}, this env has {have_stream!r}")
     for name, attr in _ENV_TENSORS.items():
         t = getattr(env, attr, None)
         arr = state.get(f"env/{name}")
@@ -77,6 +82,8 @@ def load_env_state_dict(env, state: Dict[str, object]) -> None:
         if arr is None:
             if name in ("obs_clipped", "states_clipped"):
                 continue          # the writer had no wrapper attached; the next step refills them
+            if name == "torch_rng":
+                continue          # written before the torch stream existed: the env keeps its seeded state
             raise ValueError(f"checkpoint lacks env/{name}")
         src = torch.from_numpy(np.ascontiguousarray(arr))
         if tuple(src.shape) != tuple(t.shape) or src.dtype != t.dtype:

@@ -103,6 +103,10 @@ def default_trifinger_config() -> Dict[str, Any]:
             "obs_noise_std": {"robot_q": 0.0, "robot_u": 0.0, "object_q": 0.0, "object_q_des": 0.0, "command": 0.0},
             "action_noise_std": 0.0,  # additive Gaussian on the action before clipping
         },
+        # where reset / goal samples come from: "philox" = this build's own counter stream, keyed by (seed, global env
+        # id), the same for any sharding; "torch" = the numbers the reference's own torch.rand / torch.randn calls on
+        # the CUDA device return after the same seed (one process only; env.sync_torch_generator / load_torch_generator)
+        "rng_stream": "philox",
     }
 
 

@@ -4,7 +4,8 @@
 // square root and without fast-math, so every fp32 operation below rounds exactly once, in
 // the order written — the order of the reference's ATen ops.  The only fused multiply-adds
 // are the explicit __fmaf_rn calls in norm3(), which reproduce the contraction inside
-// ATen's CPU 2-norm reduction (measured against torch 2.11; see DESIGN.md "numerics").
+// ATen's CPU 2-norm reduction (measured against torch 2.11; see DESIGN.md "numerics"), and
+// the one in torch_normal(), which reproduces the contraction in torch's CUDA Box-Muller.
 //
 // All reference paths are relative to /root/reference/leibnizgym/.
 #pragma once
@@ -260,6 +261,141 @@ __device__ __forceinline__ DrawSource make_draws(const LgParams& P, uint64_t epo
 }
 
 // ---------------------------------------------------------------------------------------
+// torch's CUDA Philox stream (LG_RNG_TORCH; SURVEY.md §D option A)
+// ---------------------------------------------------------------------------------------
+// torch.rand / torch.randn of n fp32 elements (ATen/native/cuda/DistributionTemplates.h): a grid-stride kernel of
+// g = min(SMs x threads_per_sm / 256, ceil(n / 256)) blocks of 256 threads; thread t runs curand_init(seed, t, offset)
+// and draws one Philox4x32-10 block per round, whose four words feed elements t + T (4 r + lane), T = 256 g.
+// `gmax` = SMs x (threads_per_sm / 256).  All sizes fit 32 bits: n < 18 x 2^23.
+__host__ __device__ __forceinline__ uint32_t torch_threads(uint32_t n, uint32_t gmax) {
+  const uint32_t g = (n + 255u) / 256u;
+  return 256u * (g < gmax ? g : gmax);
+}
+// how far one call of n elements advances the generator's offset (calc_execution_policy)
+__host__ __device__ __forceinline__ uint32_t torch_advance(uint32_t n, uint32_t gmax) {
+  return n == 0 ? 0u : 4u * ((n - 1u) / (4u * torch_threads(n, gmax)) + 1u);
+}
+// the Philox block element j of such a call comes from, and its lane: curand_init puts the key = seed, the
+// subsequence (thread) in the high counter words and offset / 4 + round in the low ones (curand_philox4x32_x.h)
+__device__ __forceinline__ U4 torch_block(uint64_t seed, uint64_t offset, uint32_t n, uint32_t gmax, uint32_t j, int& lane) {
+  const uint32_t T = torch_threads(n, gmax), q = j / T;
+  lane = (int)(q & 3u);
+  const uint64_t c = (offset >> 2) + (q >> 2);
+  return philox4x32_10(U4{(uint32_t)c, (uint32_t)(c >> 32), j - q * T, 0u}, (uint32_t)seed, (uint32_t)(seed >> 32));
+}
+constexpr float kTwoPow32Inv = 2.3283064365386963e-10f;         // CURAND_2POW32_INV = 2^-32
+constexpr float kTwoPow32Inv2Pi = kTwoPow32Inv * 6.2831855f;       // CURAND_2POW32_INV_2PI (exact product)
+__device__ __forceinline__ uint32_t u4_lane(const U4 w, int lane) {
+  return lane == 0 ? w.x : lane == 1 ? w.y : lane == 2 ? w.z : w.w;
+}
+// curand_uniform (x 2^-32 + 2^-33, in (0, 1]), then uniform_kernel's `v * 1 + 0` and `v == 1 ? 0 : v`
+__device__ __forceinline__ float torch_uniform(uint32_t x) {
+  const float v = (float)x * kTwoPow32Inv + kTwoPow32Inv * 0.5f;
+  return v == 1.0f ? 0.0f : v;
+}
+// curand_normal4: _curand_box_muller on words (0, 1) and (2, 3), lane 0 / 2 = s sin v, lane 1 / 3 = s cos v.  torch's
+// kernels are compiled with contraction on: v = y (2 pi 2^-32) + pi 2^-32 is one FFMA there (u's product is exact,
+// logf's code does not depend on contraction, __sincosf is MUFU.SIN / MUFU.COS).
+__device__ __forceinline__ float torch_normal(const U4 w, int lane) {
+  const uint32_t a = lane < 2 ? w.x : w.z, b = lane < 2 ? w.y : w.w;
+  const float u = (float)a * kTwoPow32Inv + kTwoPow32Inv * 0.5f;
+  const float v = __fmaf_rn((float)b, kTwoPow32Inv2Pi, kTwoPow32Inv2Pi * 0.5f);
+  const float s = sqrtf(-2.0f * logf(u));
+  float sn, cs;
+  __sincosf(v, &sn, &cs);
+  return (lane & 1) ? cs * s : sn * s;
+}
+
+// The reference's calls of one _reset_impl (goal_only = false) or _goal_reset_impl (true) for a list of k envs, in
+// its order (SURVEY.md §A.5, oracle/trifinger_oracle.py), and the canonical columns each one fills:
+//   rand(k, 18) -> u0..17 (robot, random reset) | rand(k) x 3 -> u18, u19, u20 (object, random reset)
+//   goal: rand(k) -> u21, u22 (difficulties -1, 1, 3, 4, 5), u23 (-1, 3, 4, 5); randn(k, 4) -> n0..3 (4, 5, 6);
+//         rotation: randn(k, 3) -> n4..6, randn(k, 1) -> n7
+// Column c of a call of width w is element rank x w + c of it.
+struct TorchPlan {
+  uint32_t k, gmax;
+  bool robot, object, goal_uv, goal_w, goal_n, rot;
+  __host__ __device__ uint32_t adv(uint32_t w) const { return torch_advance(k * w, gmax); }
+  __host__ __device__ uint32_t goal_base() const { return (robot ? adv(18) : 0u) + (object ? 3u * adv(1) : 0u); }
+  __host__ __device__ uint32_t goal_uniforms() const { return (goal_uv ? 2u : 0u) + (goal_w ? 1u : 0u); }
+  __host__ __device__ uint32_t total() const {   // the whole list's advance
+    return k == 0 ? 0u : goal_base() + goal_uniforms() * adv(1) + (goal_n ? adv(4) : 0u) + (rot ? adv(3) + adv(1) : 0u);
+  }
+};
+__host__ __device__ __forceinline__ TorchPlan torch_plan(const LgParams& P, uint32_t k, bool goal_only) {
+  TorchPlan p;
+  const int d = P.task_difficulty;
+  p.k = k;
+  p.gmax = (uint32_t)P.sm_count * ((uint32_t)P.threads_per_sm / 256u);
+  p.robot = !goal_only && P.robot_reset == LG_RESET_RANDOM;
+  p.object = !goal_only && P.object_reset == LG_RESET_RANDOM;
+  p.goal_uv = d == -1 || d == 1 || d == 3 || d == 4 || d == 5;
+  p.goal_w = d == -1 || d == 3 || d == 4 || d == 5;
+  p.goal_n = d == 4 || d == 5 || d == 6;
+  p.rot = P.goal_rotation != 0;
+  return p;
+}
+
+// DrawSource of the torch stream: the same interface, the canonical columns of ONE env (its rank in the list) drawn
+// where the reference's calls would have put them.  One Philox evaluation per column (against one per four columns
+// in the own stream); columns that no call fills read 0 and are never used by the samplers.
+struct TorchDraws {
+  uint64_t seed, base;   // base: the offset of the list's first call
+  TorchPlan p;
+  uint32_t rank;
+  __device__ float uniform_col(int c) const {
+    uint64_t o = base;
+    uint32_t n = p.k, e = rank;
+    if (c < 18) {
+      if (!p.robot) return 0.0f;
+      n = 18u * p.k; e = rank * 18u + (uint32_t)c;
+    } else if (c < 21) {
+      if (!p.object) return 0.0f;
+      o += (p.robot ? p.adv(18) : 0u) + (uint32_t)(c - 18) * p.adv(1);
+    } else {
+      if (c < 23 ? !p.goal_uv : !p.goal_w) return 0.0f;
+      o += p.goal_base() + (uint32_t)(c - 21) * p.adv(1);
+    }
+    int lane;
+    const U4 w = torch_block(seed, o, n, p.gmax, e, lane);
+    return torch_uniform(u4_lane(w, lane));
+  }
+  __device__ float normal_col(int c) const {
+    uint64_t o = base + p.goal_base() + p.goal_uniforms() * p.adv(1);
+    uint32_t n, e;
+    if (c < 4) {
+      if (!p.goal_n) return 0.0f;
+      n = 4u * p.k; e = rank * 4u + (uint32_t)c;
+    } else {
+      if (!p.rot) return 0.0f;
+      if (p.goal_n) o += p.adv(4);
+      if (c < 7) { n = 3u * p.k; e = rank * 3u + (uint32_t)(c - 4); }
+      else { o += p.adv(3); n = p.k; e = rank; }
+    }
+    int lane;
+    const U4 w = torch_block(seed, o, n, p.gmax, e, lane);
+    return torch_normal(w, lane);
+  }
+  __device__ void uniform4(int b, float out[4]) const {
+#pragma unroll 1
+    for (int q = 0; q < 4; ++q) out[q] = uniform_col(4 * b + q);
+  }
+  __device__ void normal4(bool first, float out[4]) const {
+#pragma unroll 1
+    for (int q = 0; q < 4; ++q) out[q] = normal_col((first ? 0 : 4) + q);
+  }
+};
+
+__device__ __forceinline__ TorchDraws make_torch_draws(const LgParams& P, uint64_t seed, uint64_t base, uint32_t k,
+                                                       bool goal_only, int64_t rank) {
+  TorchDraws d;
+  d.seed = seed; d.base = base;
+  d.p = torch_plan(P, k, goal_only);
+  d.rank = (uint32_t)rank;
+  return d;
+}
+
+// ---------------------------------------------------------------------------------------
 // samplers (envs/trifinger/sample.py)
 // ---------------------------------------------------------------------------------------
 // random_xy: r = sqrt(u0) * R, theta = 2 pi u1 (sample.py:22-34)
@@ -305,7 +441,8 @@ __device__ __forceinline__ void sample_goal_position(const LgParams& P, const fl
   }
   pos[0] = x; pos[1] = y; pos[2] = z;
 }
-__device__ __forceinline__ void sample_goal_orientation(const LgParams& P, const DrawSource dr, float yaw_u, float quat[4],
+template <class D>
+__device__ __forceinline__ void sample_goal_orientation(const LgParams& P, const D dr, float yaw_u, float quat[4],
                                                         float angvel[3]) {
   const int d = P.task_difficulty;
   Quat q{0.0f, 0.0f, 0.0f, 1.0f};
@@ -330,8 +467,10 @@ __device__ __forceinline__ void sample_goal_orientation(const LgParams& P, const
 
 // Write the sampled goal into the goal buffers and the goal actor's root row (trifinger_env.py:1248-1265):
 // `half` 0 = position (+ the row's linear velocity), 1 = orientation and angular velocity, 2 = both.
+// D: DrawSource (own stream, injected columns) or TorchDraws.
+template <class D>
 __device__ __noinline__ void apply_goal_sample(const LgParams& P, const LgSimState& S, const LgBuffers& B,
-                                               int64_t e, const DrawSource dr, int half = 2) {
+                                               int64_t e, const D dr, int half = 2) {
   float* gp = B.goal_pose + e * 7;
   float* gm = B.goal_movement + e * 6;
   float* row = S.root_state + ((int64_t)P.actors_per_env * e + P.goal_slot) * 13;
@@ -371,8 +510,9 @@ constexpr int kResetSubtasks = 10;
 // from which the torque is computed right afterwards).
 // Out of line on purpose: the fused kernel reaches it from several call sites behind a block-uniform branch that most
 // tiles never take; one copy keeps the kernel's hot path (no resets) small enough to sit in the instruction cache.
+template <class D>
 __device__ __noinline__ void reset_subtask(const LgParams& P, const LgSimState& S, const LgBuffers& B, int64_t e,
-                                           int sub, const DrawSource dr, bool goal_reset_follows,
+                                           int sub, const D dr, bool goal_reset_follows,
                                            float* dof_mirror = nullptr, bool clear_flag = true) {
   if (sub < 5) {
     if (P.robot_reset == LG_RESET_NONE) return;
@@ -436,8 +576,9 @@ __device__ __noinline__ void reset_subtask(const LgParams& P, const LgSimState& 
 }
 
 // all of it for one env, in the reference's order (hooks on explicit id lists)
+template <class D>
 __device__ __forceinline__ void reset_one_env(const LgParams& P, const LgSimState& S, const LgBuffers& B,
-                                              int64_t e, const DrawSource dr) {
+                                              int64_t e, const D dr) {
   reset_subtask(P, S, B, e, 7, dr, false);
   for (int sub = 0; sub < kResetSubtasks; ++sub)
     if (sub != 7) reset_subtask(P, S, B, e, sub, dr, false);

@@ -258,6 +258,7 @@ size_t lg_struct_size(int which) {
     case 3: return sizeof(LgControl);
     case 4: return sizeof(LgRewardTerm);
     case 5: return sizeof(LgHostStep);
+    case 6: return sizeof(LgTorchRng);
     default: return 0;
   }
 }
@@ -286,6 +287,14 @@ int lg_init_history(const LgParams* P, const LgSimState* S, const LgBuffers* B, 
 }
 
 namespace {
+int check_torch_rng(const LgParams* P, const LgBuffers* B) {
+  if (!B->torch_rng) return fail(LG_ERR_BAD_ARG, "rng_stream LG_RNG_TORCH needs LgBuffers.torch_rng");
+  if (P->inject_draws) return fail(LG_ERR_BAD_ARG, "rng_stream LG_RNG_TORCH draws torch's stream: injected draws are not read");
+  if (P->sm_count <= 0 || P->threads_per_sm < 256) return fail(LG_ERR_BAD_ARG, "rng_stream LG_RNG_TORCH needs sm_count and threads_per_sm");
+  if (P->env_offset != 0 || P->global_num_envs != P->num_envs)
+    return fail(LG_ERR_BAD_ARG, "rng_stream LG_RNG_TORCH draws the stream of one process over all envs: no sharding");
+  return LG_OK;
+}
 int launch_pre(const LgParams* P, const LgSimState* S, const LgBuffers* B, const float* action_in, void* stream,
                bool chained, bool exclusive_sm) {
   if (int rc = validate(P, S, B, false)) return rc;
@@ -297,6 +306,18 @@ int launch_pre(const LgParams* P, const LgSimState* S, const LgBuffers* B, const
   const int tiles = (int)lg_scan_tiles(P->num_envs);
   if (!aligned16(action_in)) return fail(LG_ERR_BAD_ARG, "action_in must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
+  const bool torch_rng = P->rng_stream == LG_RNG_TORCH;
+  if (torch_rng) {
+    if (int rc = check_torch_rng(P, B)) return rc;
+    // list lengths and base offset first, in a launch of their own: no CTA of the pass below may wait for another
+    // one's total (ticket grids are not co-resident)
+    const int64_t want = (P->num_envs + 16 * lg::kCountThreads - 1) / (16 * lg::kCountThreads);
+    const unsigned grid = (unsigned)(want < sm_count() ? (want > 0 ? want : 1) : sm_count());
+    lg::torch_count_kernel<<<grid, lg::kCountThreads, 0, st>>>(B->reset, B->goal_reset, B->force_reset, B->force_goal_reset,
+                                                               P->num_envs, *P, B->torch_rng);
+    if (int rc = check_launch("torch_count_kernel")) return rc;
+    chained = false;   // the pass reads what the counting launch wrote: plain stream order
+  }
   // The look-back spins on predecessor tiles, so every tile a CTA can wait for must be running: while the whole grid
   // is co-resident (lg_pre_resident_tiles) tiles are block indices; larger grids take their tiles by ticket, in
   // dispatch order.  (The post pass's CTAs cannot crowd this kernel out: they are only launched once every CTA of
@@ -335,8 +356,9 @@ cudaError_t err;
     }();
     if (opt_in != cudaSuccess) return fail(LG_ERR_CUDA, std::string("pre_physics_kernel shared memory opt-in: ") + cudaGetErrorString(opt_in));
   }
-#define LG_PRE(AD, TK, MB, SP, DR) err = launch_pdl(pdl, lg::pre_physics_kernel<AD, TK, MB, SP, DR>, (unsigned)tiles, \
-                                                  SP ? lg::kPreThreads : lg::kScanThreads, DR ? dyn : 0, st, hot, *P, *S, *B)
+#define LG_PRE(AD, TK, MB, SP, DR) err = torch_rng \
+    ? launch_pdl(false, lg::pre_physics_kernel<AD, TK, MB, SP, DR, true>, (unsigned)tiles, SP ? lg::kPreThreads : lg::kScanThreads, 0, st, hot, *P, *S, *B) \
+    : launch_pdl(pdl, lg::pre_physics_kernel<AD, TK, MB, SP, DR>, (unsigned)tiles, SP ? lg::kPreThreads : lg::kScanThreads, DR ? dyn : 0, st, hot, *P, *S, *B)
   if (P->action_dim == 9) {
     if (ticket) LG_PRE(9, true, 6, false, false); else if (direct) LG_PRE(9, false, 3, true, true);
     else if (small) LG_PRE(9, false, 3, true, false); else LG_PRE(9, false, 4, true, false);
@@ -373,7 +395,14 @@ static int reset_list(const LgParams* P, const LgSimState* S, const LgBuffers* B
                       int goal_only, void* stream) {
   if (int rc = validate(P, S, B, false)) return rc;
   if (k < 0 || (k > 0 && !ids)) return fail(LG_ERR_BAD_ARG, "bad id list");
-  if (k == 0) return LG_OK;
+  if (k == 0) return LG_OK;   // the reference makes no call for an empty list: nothing is drawn
+  if (P->rng_stream == LG_RNG_TORCH) {
+    if (int rc = check_torch_rng(P, B)) return rc;
+    lg::reset_ids_kernel<true><<<(unsigned)((k + 127) / 128), 128, 0, (cudaStream_t)stream>>>(*P, *S, *B, ids, k, goal_only);
+    if (int rc = check_launch("reset_ids_kernel")) return rc;
+    lg::torch_advance_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(B->torch_rng, lg::torch_plan(*P, (uint32_t)k, goal_only != 0).total());
+    return check_launch("torch_advance_kernel");
+  }
   lg::reset_ids_kernel<<<(unsigned)((k + 127) / 128), 128, 0, (cudaStream_t)stream>>>(*P, *S, *B, ids, k, goal_only);
   if (int rc = check_launch("reset_ids_kernel")) return rc;
   lg::bump_epoch_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(B->control);
@@ -384,6 +413,24 @@ int lg_reset_envs(const LgParams* P, const LgSimState* S, const LgBuffers* B, co
 }
 int lg_goal_reset_envs(const LgParams* P, const LgSimState* S, const LgBuffers* B, const int64_t* ids, int64_t k, void* stream) {
   return reset_list(P, S, B, ids, k, 1, stream);
+}
+
+int lg_torch_philox(uint64_t seed, uint64_t offset, int64_t n, int normal, float* out, void* stream) {
+  if (n < 0 || n >= (1ll << 31) || (n > 0 && !out) || (offset & 3u)) return fail(LG_ERR_BAD_ARG, "bad argument");
+  if (n == 0) return LG_OK;
+  int dev = 0, tps = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&tps, cudaDevAttrMaxThreadsPerMultiProcessor, dev) != cudaSuccess)
+    return check_launch("lg_torch_philox");
+  const uint32_t gmax = (uint32_t)sm_count() * ((uint32_t)tps / 256u);
+  lg::torch_philox_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(seed, offset, (uint32_t)n, gmax, normal, out);
+  return check_launch("torch_philox_kernel");
+}
+uint64_t lg_torch_philox_advance(int64_t n, int32_t sm_count, int32_t threads_per_sm) {
+  if (n <= 0 || sm_count <= 0 || threads_per_sm < 256) return 0;
+  // 64-bit form of lg::torch_advance (the kernels' sizes fit 32 bits; this host function takes any n)
+  const uint64_t gmax = (uint64_t)sm_count * (uint64_t)(threads_per_sm / 256), g = ((uint64_t)n + 255) / 256;
+  const uint64_t T = 256 * (g < gmax ? g : gmax);
+  return 4 * (((uint64_t)n - 1) / (4 * T) + 1);
 }
 
 int lg_pre_step(const LgParams* P, const LgSimState* S, const LgBuffers* B, void* stream) {

@@ -229,11 +229,15 @@ struct PreHot {
 // front of it itself (count_flagged_before above), so no tile waits for another one's progress; the only grid-wide
 // hand-shake left protects the clearing of flag bytes by tiles with resets (scan_readers / scan_exits, below).
 //
+// TORCH (P.rng_stream == LG_RNG_TORCH): the resets draw torch's CUDA Philox stream (TorchDraws), which needs each
+// resetting env's global rank (the lists are resolved first, as for injected draws) and the list lengths and base offset
+// of this launch, which the counting launch in front (torch_count_kernel) left in B.torch_rng.
+//
 // SPLIT = false is the same pass with ONE 128-thread group doing both chains one after the other (look-back last, when
 // every predecessor has long published): grids of many waves are bound by the rows in flight per SM, not by the length
 // of a CTA's chain, and half-idle CTAs of 256 threads cost them a third of their throughput (1 048 576 envs: 84 against
 // 54 us).  Used together with the ticket path.
-template <int A, bool TICKET, int MINB, bool SPLIT, bool DIRECT = false>
+template <int A, bool TICKET, int MINB, bool SPLIT, bool DIRECT = false, bool TORCH = false>
 __global__ void __launch_bounds__(SPLIT ? kPreThreads : kScanThreads, MINB)
 pre_physics_kernel(const __grid_constant__ PreHot H, const __grid_constant__ LgParams P,
                    const __grid_constant__ LgSimState S, const __grid_constant__ LgBuffers B) {
@@ -358,7 +362,7 @@ pre_physics_kernel(const __grid_constant__ PreHot H, const __grid_constant__ LgP
   // us/step).  A tile with resets triggers after its torque phase (below): parked CTAs next to a long reset phase
   // were measured slower (15.4 against 15.1 us/step at 30 % resets), triggering at entry likewise for larger grids.
   if (!resets) pdl_launch_dependents();
-  const bool rank_first = resets && P.inject_draws != 0;      // injected draws are indexed by compaction rank
+  const bool rank_first = resets && (TORCH || P.inject_draws != 0);   // injected / torch draws are indexed by rank
   // DIRECT: grid-wide hand-shake about the flag bytes, kept off the row group's chain (one thread of the scan group,
   // which has slack).  `scan_readers` counts the tiles whose reads of their predecessors' flag bytes have completed (the
   // values went into the counts); a tile that is going to CLEAR flag bytes (resets) first waits for all of them.
@@ -460,16 +464,27 @@ pre_physics_kernel(const __grid_constant__ PreHot H, const __grid_constant__ LgP
   // per resetting thread.
   if (resets) {
     if (full_tile && !row_group) mbar_wait(&s_mbar, 0);   // new joint rows are mirrored into the landed slab (the row group has waited)
-    const uint32_t ex_a = s_scan[2], ex_b = s_scan[3];     // meaningful with injected draws only (rank_first)
+    const uint32_t ex_a = s_scan[2], ex_b = s_scan[3];     // meaningful with injected / torch draws only (rank_first)
     const int warp = tid >> 5, lane = tid & 31;
+    uint64_t t_seed = 0, t_base = 0;
+    uint32_t t_kr = 0, t_kg = 0;
+    if constexpr (TORCH) {   // written by the counting launch, which completed before this grid started
+      t_seed = B.torch_rng->seed; t_base = B.torch_rng->launch_base;
+      t_kr = (uint32_t)B.torch_rng->launch_counts[0]; t_kg = (uint32_t)B.torch_rng->launch_counts[1];
+    }
     auto run_sub = [&](int sub, int first, int step) {
 #pragma unroll 1
       for (int r = first; r < na; r += step) {
         const int ent = s_reset_list[r], local = ent & 0x7fff;
         const int64_t env = e0 + local;
-        const DrawSource dr = make_draws(P, (uint64_t)epoch, env, kPurposeReset, B.inject_reset_u, B.inject_reset_n,
-                                         (int64_t)ex_a + r);
-        reset_subtask(P, S, B, env, sub, dr, (ent & 0x8000) != 0, s_dof + local * 18, !DIRECT);
+        if constexpr (TORCH) {
+          const TorchDraws dr = make_torch_draws(P, t_seed, t_base, t_kr, false, (int64_t)ex_a + r);
+          reset_subtask(P, S, B, env, sub, dr, (ent & 0x8000) != 0, s_dof + local * 18, !DIRECT);
+        } else {
+          const DrawSource dr = make_draws(P, (uint64_t)epoch, env, kPurposeReset, B.inject_reset_u, B.inject_reset_n,
+                                           (int64_t)ex_a + r);
+          reset_subtask(P, S, B, env, sub, dr, (ent & 0x8000) != 0, s_dof + local * 18, !DIRECT);
+        }
       }
     };
     // Work items = (sub-task, chunk of 32 listed envs).  The four long sub-tasks (object position 5 / yaw 8, goal
@@ -492,10 +507,16 @@ pre_physics_kernel(const __grid_constant__ PreHot H, const __grid_constant__ LgP
 #pragma unroll 1
       for (int r = t2; r < nb; r += NT / 2) {
         const int64_t env = e0 + s_goal_list[r];
-        const DrawSource dr = make_draws(P, (uint64_t)epoch, env, kPurposeGoal, B.inject_goal_u, B.inject_goal_n,
-                                         (int64_t)ex_b + r);
         if (!DIRECT && half == 0) B.goal_reset[env] = 0;  // trifinger_env.py:427
-        apply_goal_sample(P, S, B, env, dr, half);
+        if constexpr (TORCH) {   // the goal-reset list draws after the whole reset list's calls
+          const TorchDraws dr = make_torch_draws(P, t_seed, t_base + torch_plan(P, t_kr, false).total(), t_kg, true,
+                                                 (int64_t)ex_b + r);
+          apply_goal_sample(P, S, B, env, dr, half);
+        } else {
+          const DrawSource dr = make_draws(P, (uint64_t)epoch, env, kPurposeGoal, B.inject_goal_u, B.inject_goal_n,
+                                           (int64_t)ex_b + r);
+          apply_goal_sample(P, S, B, env, dr, half);
+        }
       }
     }
     LG_TP(1, 7, tid == 0);
@@ -577,28 +598,95 @@ compact_kernel(const uint8_t* __restrict__ mask, int64_t n, int64_t* __restrict_
   if (f) ids[(int64_t)ex_a + t.rank_a] = e;
 }
 
-// hooks on explicit id lists
+// LG_RNG_TORCH, in front of the pre-physics pass: the lengths of both lists (flags OR forced masks), and the base
+// offset of the launch; advances the generator by all of the launch's calls.  No CTA waits for another: the last one to
+// finish (ticket) publishes.  The pre-physics pass is launched in stream order behind it.
+constexpr int kCountThreads = 256;
+__global__ void __launch_bounds__(kCountThreads)
+torch_count_kernel(const uint8_t* __restrict__ reset, const uint8_t* __restrict__ goal, const uint8_t* __restrict__ force_reset,
+                   const uint8_t* __restrict__ force_goal, int64_t n, const __grid_constant__ LgParams P, LgTorchRng* rng) {
+  __shared__ uint32_t s_cnt[kCountThreads / 32][2];
+  __shared__ bool s_last;
+  uint32_t a = 0, b = 0;
+  for (int64_t i = (int64_t)blockIdx.x * kCountThreads + threadIdx.x; i < n; i += (int64_t)gridDim.x * kCountThreads) {
+    a += (reset[i] | (force_reset ? force_reset[i] : 0)) != 0;
+    b += (goal[i] | (force_goal ? force_goal[i] : 0)) != 0;
+  }
+  a = __reduce_add_sync(0xffffffffu, a);
+  b = __reduce_add_sync(0xffffffffu, b);
+  if ((threadIdx.x & 31) == 0) { s_cnt[threadIdx.x >> 5][0] = a; s_cnt[threadIdx.x >> 5][1] = b; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    a = b = 0;
+    for (int w = 0; w < kCountThreads / 32; ++w) { a += s_cnt[w][0]; b += s_cnt[w][1]; }
+    if (a) atomicAdd(&rng->acc[0], a);
+    if (b) atomicAdd(&rng->acc[1], b);
+    __threadfence();
+    s_last = atomicAdd(&rng->ticket, 1u) == gridDim.x - 1;
+  }
+  __syncthreads();
+  if (s_last && threadIdx.x == 0) {
+    __threadfence();
+    const uint32_t kr = ld_volatile_u32(&rng->acc[0]), kg = ld_volatile_u32(&rng->acc[1]);
+    const uint64_t base = rng->offset;
+    rng->launch_base = base;
+    rng->launch_counts[0] = (int32_t)kr; rng->launch_counts[1] = (int32_t)kg;
+    rng->offset = base + torch_plan(P, kr, false).total() + torch_plan(P, kg, true).total();
+    rng->acc[0] = 0; rng->acc[1] = 0; rng->ticket = 0;
+  }
+}
+
+// torch.rand(n) / torch.randn(n) as the batched primitive lg_torch_philox: one element per thread
+__global__ void torch_philox_kernel(uint64_t seed, uint64_t offset, uint32_t n, uint32_t gmax, int normal, float* out) {
+  const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= n) return;
+  int lane;
+  const U4 w = torch_block(seed, offset, n, gmax, j, lane);
+  out[j] = normal ? torch_normal(w, lane) : torch_uniform(u4_lane(w, lane));
+}
+
+// the hooks' torch stream: the list's calls were drawn from the offset the launch read; advance it past them
+__global__ void torch_advance_kernel(LgTorchRng* rng, uint64_t adv) { rng->offset += adv; }
+
+// hooks on explicit id lists: what one listed env gets, for either draw source
+template <class D>
+__device__ __forceinline__ void hook_goal_env(const LgParams& P, const LgSimState& S, const LgBuffers& B, int64_t e,
+                                              int64_t j, const D dr) {
+  B.goal_reset[e] = 0;
+  apply_goal_sample(P, S, B, e, dr);
+  if (B.goal_root_indices) B.goal_root_indices[j] = (int32_t)(P.actors_per_env * e) + P.goal_slot;
+}
+template <class D>
+__device__ __forceinline__ void hook_reset_env(const LgParams& P, const LgSimState& S, const LgBuffers& B, int64_t e,
+                                               int64_t j, const D dr) {
+  reset_one_env(P, S, B, e, dr);
+  const int32_t base = (int32_t)(P.actors_per_env * e);
+  if (B.robot_indices) B.robot_indices[j] = base + P.robot_slot;
+  if (B.reset_root_indices) {
+    B.reset_root_indices[3 * j] = base + P.robot_slot;
+    B.reset_root_indices[3 * j + 1] = base + P.object_slot;
+    B.reset_root_indices[3 * j + 2] = base + P.goal_slot;
+  }
+}
+template <bool TORCH = false>
 __global__ void reset_ids_kernel(const __grid_constant__ LgParams P, const LgSimState S, const LgBuffers B,
                                  const int64_t* __restrict__ ids, int64_t k, int goal_only) {
   const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (j < k) {
+  if constexpr (TORCH) {   // the list's rank j is the env's index in the reference's calls
+    if (j >= k) return;
+    const int64_t e = ids[j];
+    const TorchDraws dr = make_torch_draws(P, B.torch_rng->seed, B.torch_rng->offset, (uint32_t)k, goal_only != 0, j);
+    if (goal_only) hook_goal_env(P, S, B, e, j, dr);
+    else hook_reset_env(P, S, B, e, j, dr);
+  } else if (j < k) {
     const int64_t e = ids[j];
     const uint64_t epoch = B.control->rng_epoch | (1ull << 63);  // never collides with the fused path's epochs
     if (goal_only) {
       const DrawSource dr = make_draws(P, epoch, e, kPurposeGoal, B.inject_goal_u, B.inject_goal_n, j);
-      B.goal_reset[e] = 0;
-      apply_goal_sample(P, S, B, e, dr);
-      if (B.goal_root_indices) B.goal_root_indices[j] = (int32_t)(P.actors_per_env * e) + P.goal_slot;
+      hook_goal_env(P, S, B, e, j, dr);
     } else {
       const DrawSource dr = make_draws(P, epoch, e, kPurposeReset, B.inject_reset_u, B.inject_reset_n, j);
-      reset_one_env(P, S, B, e, dr);
-      const int32_t base = (int32_t)(P.actors_per_env * e);
-      if (B.robot_indices) B.robot_indices[j] = base + P.robot_slot;
-      if (B.reset_root_indices) {
-        B.reset_root_indices[3 * j] = base + P.robot_slot;
-        B.reset_root_indices[3 * j + 1] = base + P.object_slot;
-        B.reset_root_indices[3 * j + 2] = base + P.goal_slot;
-      }
+      hook_reset_env(P, S, B, e, j, dr);
     }
   }
 }

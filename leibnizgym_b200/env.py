@@ -243,6 +243,9 @@ class TrifingerEnv(IsaacEnvBase):
         self.rank, self.world_size = int(rank), int(world_size)
         if self._global_N % self.world_size != 0:
             raise ValueError("num_instances must be divisible by world_size")
+        if cfg.get("rng_stream", "philox") == "torch" and self.world_size > 1:
+            # the reference is one process drawing for all envs: a per-shard copy of its stream is no run of it
+            raise ValueError('rng_stream "torch" draws the stream of one process over all envs: world_size must be 1')
         local_n = self._global_N // self.world_size
         self._env_offset = self.rank * local_n
         cfg["num_instances"] = local_n  # buffers hold the local shard; config['global_num_instances'] keeps the total
@@ -305,9 +308,13 @@ class TrifingerEnv(IsaacEnvBase):
         self._scan_status = torch.zeros(int(self._lib.lg_scan_tiles(N)), device=dev, dtype=torch.int64)
         self._control = torch.zeros(4, device=dev, dtype=torch.int64)  # LgControl, 32 bytes
         self._inject = {}
+        # LgTorchRng, 48 bytes: torch's CUDA generator state (seed, offset) for "rng_stream": "torch", and workspace
+        self._torch_rng = torch.zeros(6, device=dev, dtype=torch.int64)
+        props = torch.cuda.get_device_properties(dev)
         self._P = build_params(self.config, N, env_offset=self._env_offset, global_num_envs=self._global_N,
                                fingertip_bodies=s.fingertip_bodies, bodies_per_env=s.bodies_per_env,
-                               actors_per_env=s.actors_per_env, slots=s.slots)
+                               actors_per_env=s.actors_per_env, slots=s.slots, sm_count=props.multi_processor_count,
+                               threads_per_sm=props.max_threads_per_multi_processor)
         tab = np.zeros((4, nat.LG_MAX_STATE_DIM), np.float32)
         tab[0], tab[1], tab[2] = self._P.scale_centre, self._P.scale_span, self._P.scale_rcp
         tab[3] = self._P.dr_sigma
@@ -353,6 +360,7 @@ class TrifingerEnv(IsaacEnvBase):
         b.reset_ids, b.goal_reset_ids, b.counts = p(self._reset_ids), p(self._goal_reset_ids), p(self._counts)
         b.robot_indices, b.reset_root_indices, b.goal_root_indices = p(self._robot_indices), p(self._reset_root_indices), p(self._goal_root_indices)
         b.scan_status, b.control = p(self._scan_status), p(self._control)
+        b.torch_rng = p(self._torch_rng)
         b.scale_table = p(self._scale_table)
         b.reward_coef = p(self._reward_coef)
         self._B = b
@@ -433,6 +441,8 @@ class TrifingerEnv(IsaacEnvBase):
     def inject_draws(self, reset=None, goal=None):
         """Test hook: the next reset / goal reset reads these (uniforms [k,24], normals [k,8])
         instead of the Philox stream; rows are indexed by ascending-id rank."""
+        if self.config["rng_stream"] == "torch" and (reset is not None or goal is not None):
+            raise ValueError('inject_draws: with rng_stream "torch" the resets draw torch\'s stream, not injected arrays')
         dev = self._torch_device
         self._inject = {}
         for kind, pair in (("reset", reset), ("goal", goal)):
@@ -460,6 +470,46 @@ class TrifingerEnv(IsaacEnvBase):
         else:
             self._inject.pop(kind, None)
         self._apply_injection()
+
+    # -- torch's CUDA generator ("rng_stream": "torch") ------------------------------------------------
+    def seed(self, seed: int = None):
+        """ref env_base.py:312-320; with "rng_stream": "torch" the env's copy of torch's CUDA generator starts where
+        `torch.manual_seed(seed)` leaves the real one: that seed, offset 0.  Without a seed it takes the real one's state."""
+        IsaacEnvBase.seed(seed)
+        if getattr(self, "_torch_rng", None) is None:
+            return
+        if seed is None:
+            self.load_torch_generator()
+        else:
+            self._set_torch_rng(int(seed) & 0xFFFFFFFFFFFFFFFF, 0)
+
+    def _torch_generator(self) -> torch.Generator:
+        return torch.cuda.default_generators[self._torch_device.index if self._torch_device.index is not None
+                                             else torch.cuda.current_device()]
+
+    def _set_torch_rng(self, seed: int, offset: int):
+        """Two fill launches with the values as kernel arguments: stream-ordered, no host synchronisation."""
+        as_i64 = lambda v: v - (1 << 64) if v >= (1 << 63) else v  # noqa: E731  (uint64 bits in an int64 tensor)
+        self._torch_rng[0].fill_(as_i64(seed))
+        self._torch_rng[1].fill_(as_i64(offset))
+
+    def torch_rng_state(self) -> Tuple[int, int]:
+        """(seed, Philox offset) of the env's stream; synchronises the host."""
+        seed, offset = (int(v) & 0xFFFFFFFFFFFFFFFF for v in self._torch_rng[:2].tolist())
+        return seed, offset
+
+    def sync_torch_generator(self):
+        """Writes the env's stream state into torch's default CUDA generator of the env's device (one host sync): a
+        loop that draws its own numbers from that generator between steps then continues the reference's stream."""
+        seed, offset = self.torch_rng_state()
+        g = self._torch_generator()
+        g.manual_seed(seed)
+        g.set_offset(offset)
+
+    def load_torch_generator(self):
+        """The other way: the env's stream continues from torch's default CUDA generator (no device sync)."""
+        g = self._torch_generator()
+        self._set_torch_rng(int(g.initial_seed()), int(g.get_offset()))
 
     # -- public surface -------------------------------------------------------------------------
     def _frame_count(self) -> int:

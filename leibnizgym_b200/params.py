@@ -118,8 +118,9 @@ def _fill_terms(p: nat.LgParams, cfg_terms: dict) -> None:
 
 def build_params(cfg: dict, num_local_envs: int, env_offset: int = 0, global_num_envs: int | None = None,
                  fingertip_bodies=(6, 11, 16), bodies_per_env: int = 20, actors_per_env: int = 4,
-                 slots=(0, 2, 3)) -> nat.LgParams:
-    """Flattens a resolved config (config.resolve_config) into the kernel parameter block."""
+                 slots=(0, 2, 3), sm_count: int = 0, threads_per_sm: int = 0) -> nat.LgParams:
+    """Flattens a resolved config (config.resolve_config) into the kernel parameter block.  `sm_count` /
+    `threads_per_sm`: the device's, which fix torch's launch grid and so its stream ("rng_stream": "torch")."""
     mode = cfg["command_mode"]
     if mode not in nat.CMD_MODES:
         raise ValueError(f"Invalid command mode. Input: {mode} not in ['torque', 'position'].")
@@ -133,6 +134,10 @@ def build_params(cfg: dict, num_local_envs: int, env_offset: int = 0, global_num
     if o_kind not in nat.RESET_KINDS:
         raise ValueError(f"Invalid object initial state distribution. Input: {o_kind} "
                          "not in [`default`, `random`, `none`].")
+
+    stream = cfg.get("rng_stream", "philox")
+    if stream not in nat.RNG_STREAMS:
+        raise ValueError(f"Invalid rng_stream. Input: {stream!r} not in {list(nat.RNG_STREAMS)}.")
 
     p = nat.LgParams()
     p.num_envs = int(num_local_envs)
@@ -196,6 +201,8 @@ def build_params(cfg: dict, num_local_envs: int, env_offset: int = 0, global_num
             for c in range(a, b):
                 p.dr_sigma[c] = float(std.get(name, 0.0))
     p.seed = int(cfg["seed"]) & 0xFFFFFFFFFFFFFFFF
+    p.rng_stream = nat.RNG_STREAMS[stream]
+    p.sm_count, p.threads_per_sm = int(sm_count), int(threads_per_sm)
     p.inject_draws = 0
     p.use_device_clock = 0
     p.fuse_bookkeeping = 1
