@@ -711,19 +711,26 @@ post_physics_kernel(const __grid_constant__ LgParams P, const __grid_constant__ 
       for (int k = 0; k < EP; ++k) {
         const float sv = div_by_const(v[k] - centre, half_span, rcp_half, amax);
         float ov = sv;
-        if (noisy && to_obs) {
+        // sigma = 0 columns (and non-observation lanes) skip it: their noise row is never generated, and 0 * a stale
+        // inf / NaN left in shared memory by an earlier CTA would be NaN
+        if (noisy && sigma != 0.0f) {
           const float n0 = s_noise[dcol][env_first + k];   // generated before the barrier, see above
           ov = div_by_const((v[k] + sigma * n0) - centre, half_span, rcp_half, amax);
         }
         if (FULLC || k < cnt) emit_one(k, sv, ov);
       }
-      if (!(amax < kDivSafeMax)) {  // cold: a numerator left the fast division's window: IEEE division (no noise)
+      if (!(amax < kDivSafeMax)) {  // cold: a numerator left the fast division's window: IEEE division
         const float c0 = P.scale_centre[dcol], span = P.scale_span[dcol];
 #pragma unroll
         for (int k = 0; k < EP; ++k) {   // unrolled: v[] must stay in registers
           if (FULLC || k < cnt) {
             const float x = P.normalize_obs ? __fdiv_rn(2.0f * (v[k] - c0), span) : v[k];
-            emit_one(k, x, x);
+            float xo = x;
+            if (noisy && sigma != 0.0f) {   // the lane's finite envs keep their noise: bit-identical to the fast path
+              const float vn = v[k] + sigma * s_noise[dcol][env_first + k];
+              xo = P.normalize_obs ? __fdiv_rn(2.0f * (vn - c0), span) : vn;
+            }
+            emit_one(k, x, xo);
           }
         }
       }

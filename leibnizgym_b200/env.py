@@ -171,6 +171,12 @@ class IsaacEnvBase:
     def step(self, action: Union[np.ndarray, torch.Tensor]) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, dict]:
         """Generic hook-by-hook sequencing (ref env_base.py:345-401); TrifingerEnv overrides it
         with the fused two-launch version."""
+        dr = self.config.get("domain_randomization") or {}
+        if dr.get("activate") and float(dr.get("action_noise_std", 0.0)) != 0.0:
+            # the action noise is keyed by the compaction epoch, which only the fused pre-physics pass advances: hook
+            # steps would store the raw action and, if they drew at all, draw the same noise every step
+            raise ValueError("domain_randomization.action_noise_std > 0 is applied by the fused step only: "
+                             "step with TrifingerEnv.step, not the hook-by-hook IsaacEnvBase.step")
         self._step_info = {}
         action = self._check_action(action)
         self._action_buf.copy_(action)
