@@ -75,6 +75,16 @@ enum LgStat {
   LG_STAT_DONES = 12            /* count of dones                                      */
 };
 
+/* Extension (no reference code): slots of LgBuffers.episode_stats, the episodes that ended by a reset (any route but
+ * a goal-only reset) and were first seen by this lg_post_physics call.  Sums over the envs of this shard. */
+#define LG_NUM_EPISODE_STATS 4
+enum LgEpisodeStat {
+  LG_EPISODE_COUNT = 0,         /* finished episodes                                   */
+  LG_EPISODE_RETURN_SUM = 1,    /* sum of their returns (sum of fp32 rewards)          */
+  LG_EPISODE_LENGTH_SUM = 2,    /* sum of their lengths in steps                       */
+  LG_EPISODE_SUCCESSES = 3      /* how many ended with `_successes` set                */
+};
+
 typedef struct LgRewardTerm {
   int32_t activate;    /* RewardTerm.activate (utils/mdp.py:11-33)                        */
   int32_t _pad;
@@ -239,6 +249,15 @@ typedef struct LgBuffers {
      caller does with `env._reset_buf |= mask` between steps (tests, reset-heavy workloads), without a separate pass */
   const uint8_t* force_reset;
   const uint8_t* force_goal_reset;
+  /* optional episode statistics (extension, no reference code): all five or none.  lg_post_physics adds each env's
+     reward to its running return; every reset of an env with steps_count > 0 (lg_pre_physics, lg_reset_envs; not a
+     goal-only reset) moves the return, steps_count and _successes into the env's record and zeroes the return; the
+     first lg_post_physics after the reset adds the record into episode_stats (zeroed where step_stats is) */
+  float* episode_return;          /* [N] return of the running episode                                  */
+  float* last_episode_return;     /* [N] record of the env's last finished episode: return              */
+  int64_t* last_episode_length;   /* [N]   its length in steps (0: none finished yet)                   */
+  uint8_t* last_episode_success;  /* [N]   _successes when it ended                                      */
+  double* episode_stats;          /* [LG_NUM_EPISODE_STATS] LgEpisodeStat sums of the episodes reported  */
   LgTorchRng* torch_rng;    /* P.rng_stream == LG_RNG_TORCH: the generator state (NULL otherwise)  */
 } LgBuffers;
 
@@ -290,7 +309,8 @@ int lg_pre_physics_chained(const LgParams* P, const LgSimState* S, const LgBuffe
  * Everything after physics, one launch: _post_step (trifinger_env.py:500-559) =
  * _fill_observations_and_states (:959-1051) + six reward terms (rewards.py) + accumulation and
  * per-term means (:551-554) + __check_termination (:1053-1099), then the step counter, timeout
- * and dones of IsaacEnvBase.step (env_base.py:391-399) and the episode statistics.
+ * and dones of IsaacEnvBase.step (env_base.py:391-399) and the step statistics (plus, with
+ * LgBuffers.episode_return, the running returns and the finished-episode statistics).
  * `sched_step` is env_steps_count (env_base.py:286-289); ignored when P->use_device_clock.
  */
 int lg_post_physics(const LgParams* P, const LgSimState* S, const LgBuffers* B,

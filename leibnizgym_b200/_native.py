@@ -29,6 +29,8 @@ CMD_MODES = {"position": 0, "torque": 1, "position_impedance": 2}
 RESET_KINDS = {"none": 0, "default": 1, "random": 2}
 RNG_STREAMS = {"philox": 0, "torch": 1}
 STAT_POSITION_GOAL, STAT_ORIENTATION_GOAL, STAT_SUCCESSES, STAT_REWARD, STAT_RESETS, STAT_DONES = 7, 8, 9, 10, 11, 12
+LG_NUM_EPISODE_STATS = 4
+EPISODE_COUNT, EPISODE_RETURN_SUM, EPISODE_LENGTH_SUM, EPISODE_SUCCESSES = 0, 1, 2, 3   # LgEpisodeStat
 
 c_float_p = C.POINTER(C.c_float)
 
@@ -92,7 +94,9 @@ class LgBuffers(C.Structure):
         "term_rewards", "step_stats", "reset_ids", "goal_reset_ids", "counts",
         "robot_indices", "reset_root_indices", "goal_root_indices", "scan_status", "control", "reward_coef", "scale_table",
         "inject_reset_u", "inject_reset_n", "inject_goal_u", "inject_goal_n", "obs_bf16", "states_bf16",
-        "force_reset", "force_goal_reset", "torch_rng")]
+        "force_reset", "force_goal_reset",
+        "episode_return", "last_episode_return", "last_episode_length", "last_episode_success", "episode_stats",
+        "torch_rng")]
 
 
 class LgHostStep(C.Structure):

@@ -4,7 +4,7 @@ The reference has no resume path for the environment (SURVEY.md §5; `dump_confi
 envs/env_base.py:295-309, only writes the config).  A run of this build can stop after any step
 and continue bit-identically: the file holds the goal poses and movement, step counters, reset /
 goal-reset / success flags, the one-deep history, the last action / outputs, the per-step
-statistics, the device control block (RNG epoch of the kernel's Philox stream, frame counter,
+statistics (and, with "episode_statistics" on, the running returns and last-episode records), the device control block (RNG epoch of the kernel's Philox stream, frame counter,
 compaction epoch) and the state of the torch CUDA stream (`rng_stream` "torch": seed, offset) — plus, for `SyntheticSim`, the simulator tensors and its clock, because the
 pre-physics pass of the next step reads (and the resets wrote) simulator memory.
 
@@ -31,6 +31,10 @@ _ENV_TENSORS = {
     "applied_torque": "_applied_torque", "step_stats": "_step_stats", "control": "_control",
     "scan_status": "_scan_status", "counts": "_counts", "reset_ids": "_reset_ids", "goal_reset_ids": "_goal_reset_ids",
     "reward_coef": "_reward_coef", "torch_rng": "_torch_rng",
+    # episode statistics (absent when the extension is off)
+    "episode_return": "_episode_return", "last_episode_return": "_last_episode_return",
+    "last_episode_length": "_last_episode_length", "last_episode_success": "_last_episode_success",
+    "episode_stats": "_episode_stats",
 }
 _SIM_TENSORS = ("dof_state", "root_state", "rigid_body", "dof_force", "ft_sensors")
 
@@ -53,7 +57,7 @@ def env_state_dict(env) -> Dict[str, object]:
     out["meta"] = {
         "format": FORMAT_VERSION, "num_instances": int(env.num_instances), "global_num_instances": int(env._global_N),
         "env_offset": int(env._env_offset), "obs_dim": int(env.get_obs_dim()), "state_dim": int(env.get_state_dim()),
-        "action_dim": int(env.get_action_dim()), "sim": sim_meta, "config": json.loads(json.dumps(env.config, default=str)),
+        "action_dim": int(env.get_action_dim()), "episode_statistics": _episode_statistics(env.config), "sim": sim_meta, "config": json.loads(json.dumps(env.config, default=str)),
     }
     return out
 
@@ -74,6 +78,11 @@ def load_env_state_dict(env, state: Dict[str, object]) -> None:
     ck_stream = meta.get("config", {}).get("rng_stream", "philox")
     if ck_stream != have_stream:
         raise ValueError(f"checkpoint was written with rng_stream={ck_stream!r}, this env has {have_stream!r}")
+    # with the setting on, the running returns and records are part of the state: never drop or invent them
+    have_ep = _episode_statistics(env.config)
+    ck_ep = bool(meta.get("episode_statistics", _episode_statistics(meta.get("config", {}))))
+    if ck_ep != have_ep:
+        raise ValueError(f"checkpoint was written with episode_statistics.activate={ck_ep}, this env has {have_ep}")
     for name, attr in _ENV_TENSORS.items():
         t = getattr(env, attr, None)
         arr = state.get(f"env/{name}")
@@ -102,6 +111,10 @@ def load_env_state_dict(env, state: Dict[str, object]) -> None:
     env._clear_injection()
     env._step_info = env._make_info()
     torch.cuda.synchronize(env._torch_device)
+
+
+def _episode_statistics(config: dict) -> bool:
+    return bool((config.get("episode_statistics") or {}).get("activate", False))
 
 
 def save_env_state(env, path: str) -> str:

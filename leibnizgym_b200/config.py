@@ -107,6 +107,9 @@ def default_trifinger_config() -> Dict[str, Any]:
         # id), the same for any sharding; "torch" = the numbers the reference's own torch.rand / torch.randn calls on
         # the CUDA device return after the same seed (one process only; env.sync_torch_generator / load_torch_generator)
         "rng_stream": "philox",
+        # per-env running return and the record of each env's last finished episode (return, length, success), and
+        # per step the count / return sum / length sum / successes of the episodes that ended, in `info`
+        "episode_statistics": {"activate": False},
     }
 
 

@@ -567,6 +567,17 @@ __device__ __noinline__ void reset_subtask(const LgParams& P, const LgSimState& 
     // 6: goal position, 9: goal orientation + angular velocity
     if (!goal_reset_follows) apply_goal_sample(P, S, B, e, dr, sub == 6 ? 0 : 1);
   } else {
+    // extension (no reference code): the episode ends here.  Every reset route comes through this sub-task, before the
+    // counters are zeroed; steps_count == 0 means nothing happened since the previous reset and its record stays.
+    if (B.episode_return) {
+      const int64_t steps = B.steps_count[e];
+      if (steps > 0) {
+        B.last_episode_return[e] = B.episode_return[e];
+        B.last_episode_length[e] = steps;
+        B.last_episode_success[e] = B.successes[e];
+        B.episode_return[e] = 0.0f;
+      }
+    }
     if (clear_flag) B.reset[e] = 0;   // (the fused kernel's direct-prefix variant clears its tile's flags itself, later)
     B.steps_count[e] = 0;
     B.successes[e] = 0;

@@ -186,6 +186,11 @@ int validate(const LgParams* P, const LgSimState* S, const LgBuffers* B, bool ne
                       B->action, B->goal_pose, B->history, B->applied_torque};
   for (const void* p : al)
     if (p && !aligned16(p)) return fail(LG_ERR_BAD_ARG, "tensor base pointers must be 16-byte aligned");
+  const int episode_ptrs = (B->episode_return != nullptr) + (B->last_episode_return != nullptr) +
+                           (B->last_episode_length != nullptr) + (B->last_episode_success != nullptr) + (B->episode_stats != nullptr);
+  if (episode_ptrs != 0 && episode_ptrs != 5)
+    return fail(LG_ERR_BAD_ARG, "episode_return, last_episode_return, last_episode_length, last_episode_success and "
+                                "episode_stats go together");
   return LG_OK;
 }
 
@@ -197,6 +202,8 @@ int launch_post(const LgParams* P, const LgSimState* S, const LgBuffers* B, doub
   if (REWARD && !P->fuse_bookkeeping) {
     // stand-alone _post_step: nobody zeroed the accumulators (lg_pre_physics does in the fused sequence)
     if (cudaMemsetAsync(B->step_stats, 0, LG_NUM_STATS * sizeof(double), st) != cudaSuccess) return check_launch("memset");
+    if (B->episode_stats && cudaMemsetAsync(B->episode_stats, 0, LG_NUM_EPISODE_STATS * sizeof(double), st) != cudaSuccess)
+      return check_launch("memset");
   }
   const bool asym = P->asymmetric_obs != 0;
   const bool clip = B->obs_clipped != nullptr;
@@ -211,8 +218,10 @@ int launch_post(const LgParams* P, const LgSimState* S, const LgBuffers* B, doub
   const int E = P->action_dim == 9 ? pick_tile_envs(P->num_envs) : 32;
   const unsigned grid = (unsigned)((P->num_envs + E - 1) / E);
   cudaError_t err;
-  // rarely-used paths (DR noise, keypoint term, moving goal, bf16 copies) live in their own instantiation: switched off they cost nothing
-  const bool ext = P->dr_activate || P->goal_rotation || ((P->term_active_mask >> LG_TERM_KEYPOINT) & 1) || B->obs_bf16 || B->states_bf16;
+  // rarely-used paths (DR noise, keypoint term, moving goal, bf16 copies, episode statistics) live in their own
+  // instantiation: switched off they cost nothing
+  const bool ext = P->dr_activate || P->goal_rotation || ((P->term_active_mask >> LG_TERM_KEYPOINT) & 1) || B->obs_bf16 ||
+                   B->states_bf16 || B->episode_return;
 #define LG_X(AD, AS, CL, EE, EX) launch_pdl(pdl_mode() & 2, lg::post_physics_kernel<AD, AS, REWARD, CL, EE, EX>, grid, lg::kPostThreads, 0, st, *P, *S, *B, cf)
 #ifdef LG_FAST_BUILD
   if (ext || clip || P->action_dim != 9) return fail(LG_ERR_UNSUPPORTED, "LG_FAST_BUILD: instantiation not built");
@@ -573,6 +582,9 @@ int lg_step_host_pipelined(const LgParams* P, const LgSimState* S, const LgBuffe
     bc.steps_count += lo; bc.goal_pose += lo * 7; bc.goal_movement += lo * 6; bc.history += lo * LG_HISTORY_COLS;
     if (bc.applied_torque) bc.applied_torque += lo * 9;
     bc.term_rewards = nullptr;
+    if (bc.episode_return) {
+      bc.episode_return += lo; bc.last_episode_return += lo; bc.last_episode_length += lo; bc.last_episode_success += lo;
+    }
     if (int rc = lg_upload_sim_state(&pc, &sc, &hc, stream_up)) return rc;
     cudaEventRecord(pool.up[c], up);
     cudaStreamWaitEvent(main, pool.up[c], 0);

@@ -281,6 +281,12 @@ __device__ __noinline__ double stat_sums_fp64(float t0, float t1, float t2, floa
   }
   return mine;
 }
+// The same for one value per lane (episode returns outside the fixed-point window); every lane gets the sum.
+__device__ __noinline__ double warp_sum_fp64(float x) {
+  double acc = (double)x;
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  return acc;
+}
 
 constexpr int kCombineWarp = 3;   // the reward warp with the shortest sub-task (previous angle) also combines
 
@@ -388,7 +394,7 @@ template <int E, bool EXT>
 __device__ __forceinline__ void reward_combine(const LgParams& P, const LgBuffers& B, int64_t e0, int nvalid,
                                                const float* s_coef, const float* s_part,
                                                uint8_t in_goal_reset, uint8_t in_succ, uint8_t in_reset, int64_t in_steps,
-                                               const StatScale& stat_scale) {
+                                               float in_return, const StatScale& stat_scale) {
   const int tid = threadIdx.x;
   const int renv = tid & 31;
   asm volatile("bar.sync 1, 128;" ::: "memory");  // the other three reward warps have arrived: their results are in s_part
@@ -400,6 +406,10 @@ __device__ __forceinline__ void reward_combine(const LgParams& P, const LgBuffer
     float terms[7] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};   // per-env values of the statistics (0 beyond the tile)
     float reward = 0.0f;  // trifinger_env.py:511, :551-553 — accumulation in dict order (the extension term last)
     bool pos_ok = false, rot_ok = false, succ = false, reset = false, dn = false;
+    // extension (episode statistics): the record of an episode that ended since the previous pass (length 0: none)
+    int64_t ep_len = 0;
+    float ep_return = 0.0f;
+    bool ep_succ = false;
     if (live) {
       const int64_t e = e0 + env;
       const float dist = s_part[(4) * E + env], theta = s_part[(6) * E + env];
@@ -444,6 +454,15 @@ __device__ __forceinline__ void reward_combine(const LgParams& P, const LgBuffer
       }
       dn = reset && goal_reset;
       if (B.dones) B.dones[e] = dn;
+      // extension (no reference code): running return, and the record a reset wrote since the previous pass.  That
+      // reset zeroed the step counter, so the record is fresh exactly when in_steps == 0 and it holds an episode.
+      if (EXT && B.episode_return) {
+        B.episode_return[e] = in_return + reward;
+        if (in_steps == 0) {
+          const int64_t len = B.last_episode_length[e];
+          if (len > 0) { ep_len = len; ep_return = B.last_episode_return[e]; ep_succ = B.last_episode_success[e] != 0; }
+        }
+      }
     }
     LG_TP(0, 7, renv == 0);
     // ---- episode statistics (trifinger_env.py:554, :1067-1068, :1076, :1098-1099): per-CTA sums over the warp's
@@ -500,6 +519,27 @@ __device__ __forceinline__ void reward_combine(const LgParams& P, const LgBuffer
     if (mine == 1.2345e300) return;   // make the stamp below wait for the scaled value
 #endif
     LG_TP(0, 25, renv == 0);
+    // extension: finished episodes on the lanes after LG_STAT_DONES, by the same means — ballots and integer sums
+    // (exact), the returns in 2^-30 fixed point with the fp64 butterflies for |x| >= 2^28, inf and NaN.  A warp
+    // without fresh records adds nothing.
+    if (EXT && B.episode_stats) {
+      const unsigned m_ep = __ballot_sync(0xffffffffu, ep_len > 0);
+      if (m_ep) {
+        const unsigned m_ep_succ = __ballot_sync(0xffffffffu, ep_succ);
+        const long long len_sum = warp_sum_i64(ep_len);
+        double ret_sum;
+        if (__all_sync(0xffffffffu, fabsf(ep_return) < kStatFixMax))
+          ret_sum = i64_times_pow2(warp_sum_i64(__float2ll_rn(ep_return * kStatFixScale)), -30);
+        else
+          ret_sum = warp_sum_fp64(ep_return);   // cold
+        const int slot = env - (LG_STAT_DONES + 1);
+        double ep = (double)__popc(m_ep);
+        if (slot == LG_EPISODE_RETURN_SUM) ep = ret_sum;
+        if (slot == LG_EPISODE_LENGTH_SUM) ep = (double)len_sum;
+        if (slot == LG_EPISODE_SUCCESSES) ep = (double)__popc(m_ep_succ);
+        if (slot >= 0 && slot < LG_NUM_EPISODE_STATS) atomicAdd(B.episode_stats + slot, ep);
+      }
+    }
     if (env <= LG_STAT_DONES) atomicAdd(B.step_stats + env, mine);
     LG_TP(0, 8, renv == 0);
   }
@@ -597,6 +637,8 @@ post_physics_kernel(const __grid_constant__ LgParams P, const __grid_constant__ 
   // yet issued its column loads.
   asm volatile("" : "+l"(p_goal_reset), "+l"(p_succ), "+l"(p_reset), "+l"(p_steps));
   if (rlive && rw == kCombineWarp) { in_goal_reset = *p_goal_reset; in_succ = *p_succ; in_reset = *p_reset; in_steps = *p_steps; }
+  float in_return = 0.0f;   // extension: the env's running return (episode statistics)
+  if (EXT && REWARD && rlive && rw == kCombineWarp && B.episode_return) in_return = B.episode_return[e0 + renv];
   pdl_launch_dependents();  // the next kernel may start launching; it still waits for this grid to finish
   // same for the scale constants: a CTA that starts late must not wait for them before it has issued its loads
   asm volatile("" : "+f"(half_span), "+f"(rcp_half));
@@ -759,7 +801,8 @@ post_physics_kernel(const __grid_constant__ LgParams P, const __grid_constant__ 
   else emit_outputs(std::false_type{});
   LG_TP(0, 9, tid == 0);
   if (REWARD && rw == kCombineWarp)
-    reward_combine<E, EXT>(P, B, e0, nvalid, s_coef, &s_part[0][0], in_goal_reset, in_succ, in_reset, in_steps, stat_scale);
+    reward_combine<E, EXT>(P, B, e0, nvalid, s_coef, &s_part[0][0], in_goal_reset, in_succ, in_reset, in_steps, in_return,
+                           stat_scale);
   LG_TP(0, 15, tid == 128); LG_TP(0, 19, tid == 32); LG_TP(0, 20, tid == 64); LG_TP(0, 21, tid == 96);
 }
 

@@ -9,7 +9,7 @@ numbers: NCCL over NVLink on GPUs, gloo in the CPU tests.
 """
 from __future__ import annotations
 
-from typing import Dict, Tuple
+from typing import Dict, Optional, Tuple
 
 import torch
 
@@ -35,18 +35,27 @@ def stats_to_sums(step_stats: torch.Tensor, local_num_envs: int) -> torch.Tensor
 
 
 def all_reduce_stats(step_stats: torch.Tensor, local_num_envs: int, global_num_envs: int,
-                     group=None) -> torch.Tensor:
-    """Job-wide statistics vector in the same layout (means / counts) from every rank's shard vector."""
+                     group=None, episode_stats: Optional[torch.Tensor] = None):
+    """Job-wide statistics vector in the same layout (means / counts) from every rank's shard vector.
+    With `episode_stats` (a shard's LG_NUM_EPISODE_STATS sums) both go through one all-reduce and the result is the
+    pair (statistics vector, job-wide episode sums)."""
     sums = stats_to_sums(step_stats.to(torch.float64), local_num_envs)
+    n = sums.numel()
+    if episode_stats is not None:
+        sums = torch.cat([sums, episode_stats.to(device=sums.device, dtype=torch.float64)])
     if torch.distributed.is_available() and torch.distributed.is_initialized():
         torch.distributed.all_reduce(sums, op=torch.distributed.ReduceOp.SUM, group=group)
-    w = torch.ones_like(sums)
+    w = torch.ones(n, dtype=sums.dtype, device=sums.device)
     w[list(MEAN_SLOTS)] = 1.0 / float(global_num_envs)
-    return sums * w
+    if episode_stats is None:
+        return sums * w
+    return sums[:n] * w, sums[n:]
 
 
-def stats_to_info(stats: torch.Tensor, active_terms) -> Dict[str, float]:
-    """The reference's `_step_info` keys from a statistics vector."""
+def stats_to_info(stats: torch.Tensor, active_terms, episode_stats: Optional[torch.Tensor] = None) -> Dict[str, float]:
+    """The reference's `_step_info` keys from a statistics vector.  With `episode_stats` (LgEpisodeStat sums) also
+    env/episodes/{count, return_sum, length_sum, successes} and, when episodes ended, env/episodes/{mean_return,
+    mean_length, success_rate}."""
     v = stats.detach().cpu().tolist()
     out = {}
     for i, name in enumerate(nat.TERM_NAMES):
@@ -55,4 +64,11 @@ def stats_to_info(stats: torch.Tensor, active_terms) -> Dict[str, float]:
     out["env/current_position_goal/count"] = v[nat.STAT_POSITION_GOAL]
     out["env/current_orientation_goal/count"] = v[nat.STAT_ORIENTATION_GOAL]
     out["env/average_consecutive_success"] = v[nat.STAT_SUCCESSES]
+    if episode_stats is not None:
+        count, ret, length, succ = episode_stats.detach().cpu().tolist()
+        out.update({"env/episodes/count": count, "env/episodes/return_sum": ret, "env/episodes/length_sum": length,
+                    "env/episodes/successes": succ})
+        if count > 0:
+            out.update({"env/episodes/mean_return": ret / count, "env/episodes/mean_length": length / count,
+                        "env/episodes/success_rate": succ / count})
     return out

@@ -31,6 +31,9 @@ from .params import action_dim_of, action_scale, build_params, observation_scale
 from .sim import LazyCount, SyntheticSim
 from .synthetic import make_sequence
 
+# `info` keys of the episode statistics, in LgEpisodeStat order
+EPISODE_KEYS = ("env/episodes/count", "env/episodes/return_sum", "env/episodes/length_sum", "env/episodes/successes")
+
 
 class IsaacEnvBase:
     """Template-method env runtime: buffers, step sequencing, timeout bookkeeping
@@ -304,6 +307,15 @@ class TrifingerEnv(IsaacEnvBase):
         self._obs_clipped = self._states_clipped = None
         self._obs_bf16 = self._states_bf16 = None
         self._step_stats = torch.zeros(nat.LG_NUM_STATS, device=dev, dtype=torch.float64)
+        # extension: episode statistics (all five buffers or none; the kernels check)
+        self._episode_return = self._last_episode_return = self._last_episode_length = None
+        self._last_episode_success = self._episode_stats = None
+        if self.config["episode_statistics"]["activate"]:
+            self._episode_return = torch.zeros(N, device=dev, dtype=torch.float)
+            self._last_episode_return = torch.zeros(N, device=dev, dtype=torch.float)
+            self._last_episode_length = torch.zeros(N, device=dev, dtype=torch.long)
+            self._last_episode_success = torch.zeros(N, device=dev, dtype=torch.bool)
+            self._episode_stats = torch.zeros(nat.LG_NUM_EPISODE_STATS, device=dev, dtype=torch.float64)
         self._reset_ids = torch.zeros(N, device=dev, dtype=torch.long)
         self._goal_reset_ids = torch.zeros(N, device=dev, dtype=torch.long)
         self._counts = torch.zeros(2, **i32)
@@ -369,6 +381,9 @@ class TrifingerEnv(IsaacEnvBase):
         b.torch_rng = p(self._torch_rng)
         b.scale_table = p(self._scale_table)
         b.reward_coef = p(self._reward_coef)
+        b.episode_return, b.last_episode_return = p(self._episode_return), p(self._last_episode_return)
+        b.last_episode_length, b.last_episode_success = p(self._last_episode_length), p(self._last_episode_success)
+        b.episode_stats = p(self._episode_stats)
         self._B = b
         if not getattr(self, "_history_seeded", False):
             self._call("lg_init_history", self._P, self._S, self._B)  # ref trifinger_env.py:619-628
@@ -559,6 +574,32 @@ class TrifingerEnv(IsaacEnvBase):
         self._step_info = self._make_info()
         return self._obs_buf, self._reward_buf, self._dones, self._step_info
 
+    # -- episode statistics (extension, "episode_statistics": {"activate": True}; None when off) --------------------
+    # An episode ends when the env is reset by any route: timeout, a flag set between steps or a forced mask, `reset()`,
+    # `_reset_impl`.  A goal reset (success termination) does not end it.  The reset moves the running return, the
+    # step count and `_successes` into the env's record; the first step after it reports the episode in `info`
+    # (env/episodes/*).  The reset happens at the start of the next step, so an episode that times out at step t is
+    # reported by step t + 1.
+    @property
+    def episode_return(self) -> Optional[torch.Tensor]:
+        """[N] fp32: sum of the rewards of each env's running episode, success bonus included."""
+        return self._episode_return
+
+    @property
+    def last_episode_return(self) -> Optional[torch.Tensor]:
+        """[N] fp32: return of each env's last finished episode."""
+        return self._last_episode_return
+
+    @property
+    def last_episode_length(self) -> Optional[torch.Tensor]:
+        """[N] int64: its length in steps; 0 while the env has finished none."""
+        return self._last_episode_length
+
+    @property
+    def last_episode_success(self) -> Optional[torch.Tensor]:
+        """[N] bool: `_successes` at the moment it ended."""
+        return self._last_episode_success
+
     # -- checkpoint / resume (SURVEY.md §8 f4; the reference only dumps its config, env_base.py:295-309) ------
     def state_dict(self) -> dict:
         from .checkpoint import env_state_dict
@@ -591,16 +632,26 @@ class TrifingerEnv(IsaacEnvBase):
             info["env/current_position_goal/count"] = buf[nat.STAT_POSITION_GOAL]
             info["env/current_orientation_goal/count"] = buf[nat.STAT_ORIENTATION_GOAL]
             info["env/average_consecutive_success"] = buf[nat.STAT_SUCCESSES]
+            ep = self._episode_stats
+            if ep is not None:   # episodes reported by this step (sums over this shard)
+                for i, key in enumerate(EPISODE_KEYS):
+                    info[key] = ep[i]
             views = self._info_views = (buf, info)
         return dict(views[1])
 
     def global_step_info(self) -> Dict[str, float]:
         """Whole-job statistics: all-reduces the 16 shard sums (the only cross-GPU traffic of the
-        path, SURVEY.md §8e) and divides by the global env count.  Synchronises the host."""
+        path, SURVEY.md §8e) and divides by the global env count.  With episode statistics on, their four
+        sums go in the same all-reduce.  Synchronises the host."""
         from .distributed import all_reduce_stats, stats_to_info
-        stats = all_reduce_stats(self._step_stats, self.num_instances, self._global_N)
         active = [k for k, v in self.config["reward_terms"].items() if v["activate"]]
-        return stats_to_info(stats, active)
+        if self._episode_stats is None:
+            stats = all_reduce_stats(self._step_stats, self.num_instances, self._global_N)
+            return stats_to_info(stats, active)
+        # one all-reduce for both vectors; adds the job-wide episode sums and, when episodes ended, their means
+        stats, episodes = all_reduce_stats(self._step_stats, self.num_instances, self._global_N,
+                                           episode_stats=self._episode_stats)
+        return stats_to_info(stats, active, episode_stats=episodes)
 
     # -- hooks, individually callable (ref trifinger_env.py:373-559, :959-994) ---------------------
     def _reset_impl(self, instances: torch.Tensor):
