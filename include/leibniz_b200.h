@@ -85,6 +85,11 @@ enum LgEpisodeStat {
   LG_EPISODE_SUCCESSES = 3      /* how many ended with `_successes` set                */
 };
 
+/* Extension (no reference code): slots of a per-term episode return row (LgBuffers.episode_term_return,
+ * last_episode_term_return, episode_term_stats): slot k < 7 is reward term k (LgTerm order), then the success bonus. */
+#define LG_NUM_EPISODE_TERMS 8
+enum { LG_EPISODE_TERM_BONUS = 7 };
+
 typedef struct LgRewardTerm {
   int32_t activate;    /* RewardTerm.activate (utils/mdp.py:11-33)                        */
   int32_t _pad;
@@ -258,7 +263,15 @@ typedef struct LgBuffers {
   int64_t* last_episode_length;   /* [N]   its length in steps (0: none finished yet)                   */
   uint8_t* last_episode_success;  /* [N]   _successes when it ended                                      */
   double* episode_stats;          /* [LG_NUM_EPISODE_STATS] LgEpisodeStat sums of the episodes reported  */
-  LgTorchRng* torch_rng;    /* P.rng_stream == LG_RNG_TORCH: the generator state (NULL otherwise)  */
+  /* optional per-term episode returns (extension, no reference code): all three or none, and only with the five
+     episode buffers above; the two row arrays 16-byte aligned.  lg_post_physics adds each active term's value (and the
+     success bonus when it is paid) to the env's running row; the same resets that end an episode move the row into
+     the env's record and zero it; the first lg_post_physics after the reset adds the record into episode_term_stats
+     (zeroed where episode_stats is) */
+  float* episode_term_return;       /* [N, LG_NUM_EPISODE_TERMS] running episode, per term + success bonus     */
+  float* last_episode_term_return;  /* [N, LG_NUM_EPISODE_TERMS] record of the env's last finished episode     */
+  double* episode_term_stats;       /* [LG_NUM_EPISODE_TERMS] sums of the records of the episodes reported    */
+  LgTorchRng* torch_rng;   /* P.rng_stream == LG_RNG_TORCH: the generator state (NULL otherwise)  */
 } LgBuffers;
 
 int lg_version(void);

@@ -31,6 +31,9 @@ RNG_STREAMS = {"philox": 0, "torch": 1}
 STAT_POSITION_GOAL, STAT_ORIENTATION_GOAL, STAT_SUCCESSES, STAT_REWARD, STAT_RESETS, STAT_DONES = 7, 8, 9, 10, 11, 12
 LG_NUM_EPISODE_STATS = 4
 EPISODE_COUNT, EPISODE_RETURN_SUM, EPISODE_LENGTH_SUM, EPISODE_SUCCESSES = 0, 1, 2, 3   # LgEpisodeStat
+LG_NUM_EPISODE_TERMS = 8
+LG_EPISODE_TERM_BONUS = 7
+EPISODE_TERM_NAMES = TERM_NAMES + ("success_bonus",)   # slots of the per-term episode return rows
 
 c_float_p = C.POINTER(C.c_float)
 
@@ -96,6 +99,7 @@ class LgBuffers(C.Structure):
         "inject_reset_u", "inject_reset_n", "inject_goal_u", "inject_goal_n", "obs_bf16", "states_bf16",
         "force_reset", "force_goal_reset",
         "episode_return", "last_episode_return", "last_episode_length", "last_episode_success", "episode_stats",
+        "episode_term_return", "last_episode_term_return", "episode_term_stats",
         "torch_rng")]
 
 

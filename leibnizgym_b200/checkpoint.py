@@ -4,7 +4,8 @@ The reference has no resume path for the environment (SURVEY.md §5; `dump_confi
 envs/env_base.py:295-309, only writes the config).  A run of this build can stop after any step
 and continue bit-identically: the file holds the goal poses and movement, step counters, reset /
 goal-reset / success flags, the one-deep history, the last action / outputs, the per-step
-statistics (and, with "episode_statistics" on, the running returns and last-episode records), the device control block (RNG epoch of the kernel's Philox stream, frame counter,
+statistics (and, with "episode_statistics" on, the running returns and last-episode records; with
+"episode_term_returns" on, their per-term rows too), the device control block (RNG epoch of the kernel's Philox stream, frame counter,
 compaction epoch) and the state of the torch CUDA stream (`rng_stream` "torch": seed, offset) — plus, for `SyntheticSim`, the simulator tensors and its clock, because the
 pre-physics pass of the next step reads (and the resets wrote) simulator memory.
 
@@ -35,6 +36,9 @@ _ENV_TENSORS = {
     "episode_return": "_episode_return", "last_episode_return": "_last_episode_return",
     "last_episode_length": "_last_episode_length", "last_episode_success": "_last_episode_success",
     "episode_stats": "_episode_stats",
+    # per-term episode returns (absent when that extension is off)
+    "episode_term_return": "_episode_term_return", "last_episode_term_return": "_last_episode_term_return",
+    "episode_term_stats": "_episode_term_stats",
 }
 _SIM_TENSORS = ("dof_state", "root_state", "rigid_body", "dof_force", "ft_sensors")
 
@@ -57,7 +61,8 @@ def env_state_dict(env) -> Dict[str, object]:
     out["meta"] = {
         "format": FORMAT_VERSION, "num_instances": int(env.num_instances), "global_num_instances": int(env._global_N),
         "env_offset": int(env._env_offset), "obs_dim": int(env.get_obs_dim()), "state_dim": int(env.get_state_dim()),
-        "action_dim": int(env.get_action_dim()), "episode_statistics": _episode_statistics(env.config), "sim": sim_meta, "config": json.loads(json.dumps(env.config, default=str)),
+        "action_dim": int(env.get_action_dim()), "episode_statistics": _episode_statistics(env.config),
+        "episode_term_returns": _activated(env.config, "episode_term_returns"), "sim": sim_meta, "config": json.loads(json.dumps(env.config, default=str)),
     }
     return out
 
@@ -83,6 +88,10 @@ def load_env_state_dict(env, state: Dict[str, object]) -> None:
     ck_ep = bool(meta.get("episode_statistics", _episode_statistics(meta.get("config", {}))))
     if ck_ep != have_ep:
         raise ValueError(f"checkpoint was written with episode_statistics.activate={ck_ep}, this env has {have_ep}")
+    have_terms = _activated(env.config, "episode_term_returns")
+    ck_terms = bool(meta.get("episode_term_returns", _activated(meta.get("config", {}), "episode_term_returns")))
+    if ck_terms != have_terms:
+        raise ValueError(f"checkpoint was written with episode_term_returns.activate={ck_terms}, this env has {have_terms}")
     for name, attr in _ENV_TENSORS.items():
         t = getattr(env, attr, None)
         arr = state.get(f"env/{name}")
@@ -114,7 +123,11 @@ def load_env_state_dict(env, state: Dict[str, object]) -> None:
 
 
 def _episode_statistics(config: dict) -> bool:
-    return bool((config.get("episode_statistics") or {}).get("activate", False))
+    return _activated(config, "episode_statistics")
+
+
+def _activated(config: dict, key: str) -> bool:
+    return bool((config.get(key) or {}).get("activate", False))
 
 
 def save_env_state(env, path: str) -> str:

@@ -110,6 +110,9 @@ def default_trifinger_config() -> Dict[str, Any]:
         # per-env running return and the record of each env's last finished episode (return, length, success), and
         # per step the count / return sum / length sum / successes of the episodes that ended, in `info`
         "episode_statistics": {"activate": False},
+        # with "episode_statistics" on: each episode's return split by reward term plus the success bonus (running
+        # and last finished, per env), and per step the per-term sums of the episodes that ended, in `info`
+        "episode_term_returns": {"activate": False},
     }
 
 

@@ -493,6 +493,23 @@ __device__ __noinline__ void apply_goal_sample(const LgParams& P, const LgSimSta
   }
 }
 
+// extension (no reference code): the episode of env e (steps_count `steps` > 0) ends.  Its running return, length and
+// success become its record and the return is zeroed; with per-term returns, so does the running row (32 contiguous
+// bytes, two 128-bit pieces).  Out of line: the reset sub-task keeps its registers.
+__device__ __noinline__ void end_episode(const LgBuffers& B, int64_t e, int64_t steps) {
+  B.last_episode_return[e] = B.episode_return[e];
+  B.last_episode_length[e] = steps;
+  B.last_episode_success[e] = B.successes[e];
+  B.episode_return[e] = 0.0f;
+  if (B.episode_term_return) {
+    float4* run = reinterpret_cast<float4*>(B.episode_term_return + e * LG_NUM_EPISODE_TERMS);
+    float4* rec = reinterpret_cast<float4*>(B.last_episode_term_return + e * LG_NUM_EPISODE_TERMS);
+    const float4 a = run[0], b = run[1];
+    rec[0] = a; rec[1] = b;
+    run[0] = run[1] = make_float4(0.f, 0.f, 0.f, 0.f);
+  }
+}
+
 // _reset_impl for ONE env (trifinger_env.py:373-411, :1101-1192) cut into TEN independent sub-tasks, so that the
 // fused kernel can run them on different warps (uniform control flow inside a warp) instead of one long serial
 // chain per resetting env.  The draws are counter-based (or injected by column), so every sub-task fetches exactly
@@ -571,12 +588,7 @@ __device__ __noinline__ void reset_subtask(const LgParams& P, const LgSimState& 
     // counters are zeroed; steps_count == 0 means nothing happened since the previous reset and its record stays.
     if (B.episode_return) {
       const int64_t steps = B.steps_count[e];
-      if (steps > 0) {
-        B.last_episode_return[e] = B.episode_return[e];
-        B.last_episode_length[e] = steps;
-        B.last_episode_success[e] = B.successes[e];
-        B.episode_return[e] = 0.0f;
-      }
+      if (steps > 0) end_episode(B, e, steps);
     }
     if (clear_flag) B.reset[e] = 0;   // (the fused kernel's direct-prefix variant clears its tile's flags itself, later)
     B.steps_count[e] = 0;

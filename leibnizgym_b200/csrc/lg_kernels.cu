@@ -191,6 +191,15 @@ int validate(const LgParams* P, const LgSimState* S, const LgBuffers* B, bool ne
   if (episode_ptrs != 0 && episode_ptrs != 5)
     return fail(LG_ERR_BAD_ARG, "episode_return, last_episode_return, last_episode_length, last_episode_success and "
                                 "episode_stats go together");
+  const int term_ptrs = (B->episode_term_return != nullptr) + (B->last_episode_term_return != nullptr) +
+                        (B->episode_term_stats != nullptr);
+  if (term_ptrs != 0 && term_ptrs != 3)
+    return fail(LG_ERR_BAD_ARG, "episode_term_return, last_episode_term_return and episode_term_stats go together");
+  if (term_ptrs && !episode_ptrs)
+    return fail(LG_ERR_BAD_ARG, "episode_term_return needs the episode statistics buffers (episode_return, "
+                                "last_episode_return, last_episode_length, last_episode_success, episode_stats)");
+  if (term_ptrs && (!aligned16(B->episode_term_return) || !aligned16(B->last_episode_term_return)))
+    return fail(LG_ERR_BAD_ARG, "episode_term_return and last_episode_term_return must be 16-byte aligned");
   return LG_OK;
 }
 
@@ -203,6 +212,9 @@ int launch_post(const LgParams* P, const LgSimState* S, const LgBuffers* B, doub
     // stand-alone _post_step: nobody zeroed the accumulators (lg_pre_physics does in the fused sequence)
     if (cudaMemsetAsync(B->step_stats, 0, LG_NUM_STATS * sizeof(double), st) != cudaSuccess) return check_launch("memset");
     if (B->episode_stats && cudaMemsetAsync(B->episode_stats, 0, LG_NUM_EPISODE_STATS * sizeof(double), st) != cudaSuccess)
+      return check_launch("memset");
+    if (B->episode_term_stats &&
+        cudaMemsetAsync(B->episode_term_stats, 0, LG_NUM_EPISODE_TERMS * sizeof(double), st) != cudaSuccess)
       return check_launch("memset");
   }
   const bool asym = P->asymmetric_obs != 0;
@@ -584,6 +596,9 @@ int lg_step_host_pipelined(const LgParams* P, const LgSimState* S, const LgBuffe
     bc.term_rewards = nullptr;
     if (bc.episode_return) {
       bc.episode_return += lo; bc.last_episode_return += lo; bc.last_episode_length += lo; bc.last_episode_success += lo;
+    }
+    if (bc.episode_term_return) {
+      bc.episode_term_return += lo * LG_NUM_EPISODE_TERMS; bc.last_episode_term_return += lo * LG_NUM_EPISODE_TERMS;
     }
     if (int rc = lg_upload_sim_state(&pc, &sc, &hc, stream_up)) return rc;
     cudaEventRecord(pool.up[c], up);

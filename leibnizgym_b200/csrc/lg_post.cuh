@@ -51,6 +51,12 @@ __device__ __forceinline__ void bulk_store_commit_and_wait() {
   asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 }
 __device__ __forceinline__ void fence_async_proxy() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+// ---- per-thread asynchronous 16-byte copies (cp.async, SASS LDGSTS): global -> shared without a register ------------
+__device__ __forceinline__ void async_copy16(void* smem_dst, const void* gmem_src) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" :: "r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
+}
+__device__ __forceinline__ void async_copy_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+__device__ __forceinline__ void async_copy_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
 // =========================================================================================
 // post-physics: one CTA = one tile of E envs, 4 threads per env
@@ -288,6 +294,39 @@ __device__ __noinline__ double warp_sum_fp64(float x) {
   return acc;
 }
 
+// Per-term returns of the fresh records (env e, or -1: none on this lane) folded into episode_term_stats: lane
+// `tslot` keeps slot tslot, by the same means as the episode returns (2^-30 fixed point, fp64 butterflies for
+// |x| >= 2^28, inf and NaN; one decision for the warp).  Called by the combine warp when it holds fresh records; out
+// of line, so that the warp's common path keeps its registers.
+__device__ __noinline__ void episode_term_fold(const LgBuffers& B, int64_t e, int tslot) {
+  float4 ra = make_float4(0.f, 0.f, 0.f, 0.f), rb = ra;
+  if (e >= 0) {
+    const float4* rec = reinterpret_cast<const float4*>(B.last_episode_term_return + e * LG_NUM_EPISODE_TERMS);
+    ra = rec[0]; rb = rec[1];
+  }
+  const float x[LG_NUM_EPISODE_TERMS] = {ra.x, ra.y, ra.z, ra.w, rb.x, rb.y, rb.z, rb.w};
+  bool fits = true;
+#pragma unroll
+  for (int k = 0; k < LG_NUM_EPISODE_TERMS; ++k) fits = fits && fabsf(x[k]) < kStatFixMax;
+  double sum = 0.0;
+  if (__all_sync(0xffffffffu, fits)) {
+    long long fixed = 0;
+#pragma unroll
+    for (int k = 0; k < LG_NUM_EPISODE_TERMS; ++k) {
+      const long long t = warp_sum_i64(__float2ll_rn(x[k] * kStatFixScale));
+      if (tslot == k) fixed = t;
+    }
+    sum = i64_times_pow2(fixed, -30);
+  } else {
+#pragma unroll
+    for (int k = 0; k < LG_NUM_EPISODE_TERMS; ++k) {   // cold
+      const double t = warp_sum_fp64(x[k]);
+      if (tslot == k) sum = t;
+    }
+  }
+  if (tslot >= 0 && tslot < LG_NUM_EPISODE_TERMS) atomicAdd(B.episode_term_stats + tslot, sum);
+}
+
 constexpr int kCombineWarp = 3;   // the reward warp with the shortest sub-task (previous angle) also combines
 
 // ======== reward warps: lane = env, warp = sub-task (uniform control flow inside a warp) ================
@@ -394,7 +433,7 @@ template <int E, bool EXT>
 __device__ __forceinline__ void reward_combine(const LgParams& P, const LgBuffers& B, int64_t e0, int nvalid,
                                                const float* s_coef, const float* s_part,
                                                uint8_t in_goal_reset, uint8_t in_succ, uint8_t in_reset, int64_t in_steps,
-                                               float in_return, const StatScale& stat_scale) {
+                                               float in_return, float4* s_term_row, const StatScale& stat_scale) {
   const int tid = threadIdx.x;
   const int renv = tid & 31;
   asm volatile("bar.sync 1, 128;" ::: "memory");  // the other three reward warps have arrived: their results are in s_part
@@ -462,6 +501,23 @@ __device__ __forceinline__ void reward_combine(const LgParams& P, const LgBuffer
           const int64_t len = B.last_episode_length[e];
           if (len > 0) { ep_len = len; ep_return = B.last_episode_return[e]; ep_succ = B.last_episode_success[e] != 0; }
         }
+      }
+      // extension (per-term episode returns): the env's running row, staged in shared memory by the copy issued with
+      // the flag loads, takes each active term's value as the reward above took it, and the bonus when it was paid
+      if (EXT && B.episode_term_return) {
+        async_copy_wait_all();
+        float4 a = s_term_row[0], b = s_term_row[1];
+        const unsigned m = (unsigned)P.term_active_mask;
+        if (m & 1u) a.x = a.x + terms[0];
+        if (m & 2u) a.y = a.y + terms[1];
+        if (m & 4u) a.z = a.z + terms[2];
+        if (m & 8u) a.w = a.w + terms[3];
+        if (m & 16u) b.x = b.x + terms[4];
+        if (m & 32u) b.y = b.y + terms[5];
+        if (m & 64u) b.z = b.z + terms[6];
+        if (P.success_activate && goal_reset) b.w = b.w + s_coef[C_BONUS];   // goal_reset == done: the bonus was paid
+        float4* run = reinterpret_cast<float4*>(B.episode_term_return + e * LG_NUM_EPISODE_TERMS);
+        run[0] = a; run[1] = b;
       }
     }
     LG_TP(0, 7, renv == 0);
@@ -538,6 +594,8 @@ __device__ __forceinline__ void reward_combine(const LgParams& P, const LgBuffer
         if (slot == LG_EPISODE_LENGTH_SUM) ep = (double)len_sum;
         if (slot == LG_EPISODE_SUCCESSES) ep = (double)__popc(m_ep_succ);
         if (slot >= 0 && slot < LG_NUM_EPISODE_STATS) atomicAdd(B.episode_stats + slot, ep);
+        // per-term returns on the next eight lanes: one decision for the warp, as for the step statistics
+        if (B.episode_term_stats) episode_term_fold(B, ep_len > 0 ? e0 + env : -1, slot - LG_NUM_EPISODE_STATS);
       }
     }
     if (env <= LG_STAT_DONES) atomicAdd(B.step_stats + env, mine);
@@ -561,6 +619,7 @@ post_physics_kernel(const __grid_constant__ LgParams P, const __grid_constant__ 
   __shared__ float s_coef[C_COUNT];
   __shared__ float s_part[12][E];       // sub-task results of the reward warps
   __shared__ float s_noise[EXT ? L::OBS : 1][EXT ? E + 1 : 1];   // extension: standard normals of the obs columns
+  __shared__ float4 s_term_run[EXT ? 2 * E : 1];   // extension: the tile's running per-term episode returns
 
   const int tid = threadIdx.x;
   const int64_t e0 = (int64_t)blockIdx.x * E;
@@ -639,6 +698,14 @@ post_physics_kernel(const __grid_constant__ LgParams P, const __grid_constant__ 
   if (rlive && rw == kCombineWarp) { in_goal_reset = *p_goal_reset; in_succ = *p_succ; in_reset = *p_reset; in_steps = *p_steps; }
   float in_return = 0.0f;   // extension: the env's running return (episode statistics)
   if (EXT && REWARD && rlive && rw == kCombineWarp && B.episode_return) in_return = B.episode_return[e0 + renv];
+  // extension: the env's running per-term row (32 contiguous bytes) lands in shared memory by itself — no register
+  // waits for it, and the combine warp picks it up after its reward math
+  if (EXT && REWARD && rlive && rw == kCombineWarp && B.episode_term_return) {
+    const float4* row = reinterpret_cast<const float4*>(B.episode_term_return + (e0 + renv) * LG_NUM_EPISODE_TERMS);
+    async_copy16(&s_term_run[2 * renv], row);
+    async_copy16(&s_term_run[2 * renv + 1], row + 1);
+    async_copy_commit();
+  }
   pdl_launch_dependents();  // the next kernel may start launching; it still waits for this grid to finish
   // same for the scale constants: a CTA that starts late must not wait for them before it has issued its loads
   asm volatile("" : "+f"(half_span), "+f"(rcp_half));
@@ -802,7 +869,7 @@ post_physics_kernel(const __grid_constant__ LgParams P, const __grid_constant__ 
   LG_TP(0, 9, tid == 0);
   if (REWARD && rw == kCombineWarp)
     reward_combine<E, EXT>(P, B, e0, nvalid, s_coef, &s_part[0][0], in_goal_reset, in_succ, in_reset, in_steps, in_return,
-                           stat_scale);
+                           &s_term_run[EXT ? 2 * renv : 0], stat_scale);
   LG_TP(0, 15, tid == 128); LG_TP(0, 19, tid == 32); LG_TP(0, 20, tid == 64); LG_TP(0, 21, tid == 96);
 }
 

@@ -343,6 +343,7 @@ pre_physics_kernel(const __grid_constant__ PreHot H, const __grid_constant__ LgP
     // inclusive prefix, and the coefficient arithmetic below is a chain of fp64 operations.
     if (tile == 0 && gt < LG_NUM_STATS && B.step_stats) B.step_stats[gt] = 0.0;  // accumulated by lg_post_physics
     if (tile == 0 && gt < LG_NUM_EPISODE_STATS && B.episode_stats) B.episode_stats[gt] = 0.0;  // likewise (extension)
+    if (tile == 0 && gt < LG_NUM_EPISODE_TERMS && B.episode_term_stats) B.episode_term_stats[gt] = 0.0;
     if (tile == 0 && gt == kScanThreads - 1 && P.use_device_clock) {
       // device clock: advance the frame counter and publish the reward coefficients of the coming
       // post-physics pass (env_steps_count = frames x global env count, envs/env_base.py:286-289)

@@ -35,27 +35,42 @@ def stats_to_sums(step_stats: torch.Tensor, local_num_envs: int) -> torch.Tensor
 
 
 def all_reduce_stats(step_stats: torch.Tensor, local_num_envs: int, global_num_envs: int,
-                     group=None, episode_stats: Optional[torch.Tensor] = None):
+                     group=None, episode_stats: Optional[torch.Tensor] = None,
+                     episode_term_stats: Optional[torch.Tensor] = None):
     """Job-wide statistics vector in the same layout (means / counts) from every rank's shard vector.
     With `episode_stats` (a shard's LG_NUM_EPISODE_STATS sums) both go through one all-reduce and the result is the
-    pair (statistics vector, job-wide episode sums)."""
+    pair (statistics vector, job-wide episode sums).  With `episode_term_stats` too (a shard's LG_NUM_EPISODE_TERMS
+    per-term return sums) all three go through the one all-reduce and the result is the triple (statistics vector,
+    episode sums, per-term return sums)."""
+    if episode_term_stats is not None and episode_stats is None:
+        raise ValueError("episode_term_stats is reduced together with episode_stats")
     sums = stats_to_sums(step_stats.to(torch.float64), local_num_envs)
     n = sums.numel()
     if episode_stats is not None:
         sums = torch.cat([sums, episode_stats.to(device=sums.device, dtype=torch.float64)])
+    if episode_term_stats is not None:
+        sums = torch.cat([sums, episode_term_stats.to(device=sums.device, dtype=torch.float64)])
     if torch.distributed.is_available() and torch.distributed.is_initialized():
         torch.distributed.all_reduce(sums, op=torch.distributed.ReduceOp.SUM, group=group)
     w = torch.ones(n, dtype=sums.dtype, device=sums.device)
     w[list(MEAN_SLOTS)] = 1.0 / float(global_num_envs)
     if episode_stats is None:
         return sums * w
-    return sums[:n] * w, sums[n:]
+    m = n + nat.LG_NUM_EPISODE_STATS
+    if episode_term_stats is None:
+        return sums[:n] * w, sums[n:]
+    return sums[:n] * w, sums[n:m], sums[m:]
 
 
-def stats_to_info(stats: torch.Tensor, active_terms, episode_stats: Optional[torch.Tensor] = None) -> Dict[str, float]:
+def stats_to_info(stats: torch.Tensor, active_terms, episode_stats: Optional[torch.Tensor] = None,
+                  episode_term_stats: Optional[torch.Tensor] = None, episode_terms=None) -> Dict[str, float]:
     """The reference's `_step_info` keys from a statistics vector.  With `episode_stats` (LgEpisodeStat sums) also
     env/episodes/{count, return_sum, length_sum, successes} and, when episodes ended, env/episodes/{mean_return,
-    mean_length, success_rate}."""
+    mean_length, success_rate}.  With `episode_term_stats` (per-term return sums, nat.EPISODE_TERM_NAMES order) also
+    env/episodes/return_sum/<name> and, when episodes ended, env/episodes/mean_return/<name>, for the names in
+    `episode_terms` (default: all eight)."""
+    if episode_term_stats is not None and episode_stats is None:
+        raise ValueError("episode_term_stats is reported together with episode_stats")
     v = stats.detach().cpu().tolist()
     out = {}
     for i, name in enumerate(nat.TERM_NAMES):
@@ -71,4 +86,11 @@ def stats_to_info(stats: torch.Tensor, active_terms, episode_stats: Optional[tor
         if count > 0:
             out.update({"env/episodes/mean_return": ret / count, "env/episodes/mean_length": length / count,
                         "env/episodes/success_rate": succ / count})
+        if episode_term_stats is not None:
+            t = episode_term_stats.detach().cpu().tolist()
+            for i, name in enumerate(nat.EPISODE_TERM_NAMES):
+                if episode_terms is None or name in episode_terms:
+                    out[f"env/episodes/return_sum/{name}"] = t[i]
+                    if count > 0:
+                        out[f"env/episodes/mean_return/{name}"] = t[i] / count
     return out

@@ -262,6 +262,9 @@ class TrifingerEnv(IsaacEnvBase):
         A = action_dim_of(cfg["command_mode"])
         if cfg["command_mode"] not in nat.CMD_MODES:
             raise ValueError(f"Invalid command mode. Input: {cfg['command_mode']} not in ['torque', 'position'].")
+        if cfg["episode_term_returns"]["activate"] and not cfg["episode_statistics"]["activate"]:
+            raise ValueError('"episode_term_returns" needs "episode_statistics": {"activate": True}: the per-term '
+                             "returns are kept and reported with the episode statistics")
         obs_spec = {"robot_q": 9, "robot_u": 9, "object_q": 7, "object_q_des": 7, "command": A}
         if cfg["asymmetric_obs"]:
             state_spec = dict(obs_spec, object_u=6, fingertip_state=39, robot_a=9, fingertip_wrench=18)
@@ -316,6 +319,13 @@ class TrifingerEnv(IsaacEnvBase):
             self._last_episode_length = torch.zeros(N, device=dev, dtype=torch.long)
             self._last_episode_success = torch.zeros(N, device=dev, dtype=torch.bool)
             self._episode_stats = torch.zeros(nat.LG_NUM_EPISODE_STATS, device=dev, dtype=torch.float64)
+        # extension: per-term episode returns (all three or none, on top of the five above)
+        self._episode_term_return = self._last_episode_term_return = self._episode_term_stats = None
+        if self.config["episode_term_returns"]["activate"]:
+            T = nat.LG_NUM_EPISODE_TERMS
+            self._episode_term_return = torch.zeros((N, T), device=dev, dtype=torch.float)
+            self._last_episode_term_return = torch.zeros((N, T), device=dev, dtype=torch.float)
+            self._episode_term_stats = torch.zeros(T, device=dev, dtype=torch.float64)
         self._reset_ids = torch.zeros(N, device=dev, dtype=torch.long)
         self._goal_reset_ids = torch.zeros(N, device=dev, dtype=torch.long)
         self._counts = torch.zeros(2, **i32)
@@ -384,6 +394,8 @@ class TrifingerEnv(IsaacEnvBase):
         b.episode_return, b.last_episode_return = p(self._episode_return), p(self._last_episode_return)
         b.last_episode_length, b.last_episode_success = p(self._last_episode_length), p(self._last_episode_success)
         b.episode_stats = p(self._episode_stats)
+        b.episode_term_return, b.last_episode_term_return = p(self._episode_term_return), p(self._last_episode_term_return)
+        b.episode_term_stats = p(self._episode_term_stats)
         self._B = b
         if not getattr(self, "_history_seeded", False):
             self._call("lg_init_history", self._P, self._S, self._B)  # ref trifinger_env.py:619-628
@@ -600,6 +612,30 @@ class TrifingerEnv(IsaacEnvBase):
         """[N] bool: `_successes` at the moment it ended."""
         return self._last_episode_success
 
+    # -- per-term episode returns (extension, "episode_term_returns": {"activate": True}; None when off) -----------
+    # Column k < 7 of a row is reward term k (nat.TERM_NAMES), column 7 the success bonus (EPISODE_TERM_NAMES).  Each
+    # step adds what the reward added: the value of every active term (what `term_rewards` shows) and the bonus when
+    # success termination pays it; inactive terms stay 0.  The same resets that end an episode move the row into the
+    # record, and the step that reports the episode adds the record into env/episodes/return_sum/<term>.
+    EPISODE_TERM_NAMES = nat.EPISODE_TERM_NAMES
+
+    @property
+    def episode_term_return(self) -> Optional[torch.Tensor]:
+        """[N, 8] fp32: each env's running episode return split by term (EPISODE_TERM_NAMES)."""
+        return self._episode_term_return
+
+    @property
+    def last_episode_term_return(self) -> Optional[torch.Tensor]:
+        """[N, 8] fp32: the same for each env's last finished episode."""
+        return self._last_episode_term_return
+
+    def _episode_term_slots(self) -> list:
+        """Names of the slots that can be nonzero: the active reward terms and, with success termination, the bonus."""
+        names = [n for n in nat.TERM_NAMES if self.config["reward_terms"].get(n, {}).get("activate")]
+        if self.config["termination_conditions"]["success"]["activate"]:
+            names.append("success_bonus")
+        return names
+
     # -- checkpoint / resume (SURVEY.md §8 f4; the reference only dumps its config, env_base.py:295-309) ------
     def state_dict(self) -> dict:
         from .checkpoint import env_state_dict
@@ -636,22 +672,32 @@ class TrifingerEnv(IsaacEnvBase):
             if ep is not None:   # episodes reported by this step (sums over this shard)
                 for i, key in enumerate(EPISODE_KEYS):
                     info[key] = ep[i]
+            ts = self._episode_term_stats
+            if ts is not None:   # ... and their returns, split by term
+                for name in self._episode_term_slots():
+                    info[f"env/episodes/return_sum/{name}"] = ts[nat.EPISODE_TERM_NAMES.index(name)]
             views = self._info_views = (buf, info)
         return dict(views[1])
 
     def global_step_info(self) -> Dict[str, float]:
         """Whole-job statistics: all-reduces the 16 shard sums (the only cross-GPU traffic of the
         path, SURVEY.md §8e) and divides by the global env count.  With episode statistics on, their four
-        sums go in the same all-reduce.  Synchronises the host."""
+        sums (and, with per-term returns on, their eight) go in the same all-reduce.  Synchronises the host."""
         from .distributed import all_reduce_stats, stats_to_info
         active = [k for k, v in self.config["reward_terms"].items() if v["activate"]]
         if self._episode_stats is None:
             stats = all_reduce_stats(self._step_stats, self.num_instances, self._global_N)
             return stats_to_info(stats, active)
         # one all-reduce for both vectors; adds the job-wide episode sums and, when episodes ended, their means
-        stats, episodes = all_reduce_stats(self._step_stats, self.num_instances, self._global_N,
-                                           episode_stats=self._episode_stats)
-        return stats_to_info(stats, active, episode_stats=episodes)
+        if self._episode_term_stats is None:
+            stats, episodes = all_reduce_stats(self._step_stats, self.num_instances, self._global_N,
+                                               episode_stats=self._episode_stats)
+            return stats_to_info(stats, active, episode_stats=episodes)
+        stats, episodes, terms = all_reduce_stats(self._step_stats, self.num_instances, self._global_N,
+                                                  episode_stats=self._episode_stats,
+                                                  episode_term_stats=self._episode_term_stats)
+        return stats_to_info(stats, active, episode_stats=episodes, episode_term_stats=terms,
+                             episode_terms=self._episode_term_slots())
 
     # -- hooks, individually callable (ref trifinger_env.py:373-559, :959-994) ---------------------
     def _reset_impl(self, instances: torch.Tensor):
