@@ -164,6 +164,14 @@ typedef struct LgParams {
   int32_t sm_count;         /* LG_RNG_TORCH: the device's multiProcessorCount and                   */
   int32_t threads_per_sm;   /* maxThreadsPerMultiProcessor, which fix torch's launch grid           */
   int32_t _pad_tail2;
+  /* extension (no reference code): per-episode domain-randomisation offsets, drawn when an env is reset (any route
+   * but a goal-only reset) into LgBuffers.obs_bias / action_bias and added to the raw actor observation and to the
+   * action on every step of the episode.  sigma = 0 switches a column off; all zero = off.  Nonzero sigmas need
+   * dr_activate. */
+  float dr_bias_sigma[64];    /* sigma of the offset of raw obs column c (c < obs_dim = 32 + action_dim)   */
+  uint64_t dr_bias_mask;    /* bit c set exactly where dr_bias_sigma[c] != 0 (obs_dim <= 50 < 64)                  */
+  float dr_action_bias_sigma; /* sigma of the offset of every action column                                        */
+  int32_t _pad_tail3;
 } LgParams;
 
 /* Scalar coefficients of the reward terms for ONE value of env_steps_count: the Python-float
@@ -271,6 +279,16 @@ typedef struct LgBuffers {
   float* episode_term_return;       /* [N, LG_NUM_EPISODE_TERMS] running episode, per term + success bonus     */
   float* last_episode_term_return;  /* [N, LG_NUM_EPISODE_TERMS] record of the env's last finished episode     */
   double* episode_term_stats;       /* [LG_NUM_EPISODE_TERMS] sums of the records of the episodes reported    */
+  /* per-episode domain-randomisation offsets (extension, no reference code; LgParams.dr_bias_sigma /
+     dr_action_bias_sigma).  Required when the matching sigmas are nonzero, otherwise ignored.  Every reset of an env
+     (lg_pre_physics, lg_reset_envs; not a goal-only reset) redraws its rows: sigma x a standard normal of this build's
+     Philox stream keyed by (seed, global env id, epoch of the reset's own draws), never torch's stream or injected
+     draws; columns with sigma = 0 hold +0.0.  lg_post_physics / lg_fill_observations add obs_bias to the raw actor
+     observation (columns with sigma != 0 only, before the white noise); lg_pre_physics adds action_bias to the
+     incoming action before the white noise and the clamp; the rows of the envs it reset are drawn by a small launch
+     behind it. */
+  float* obs_bias;          /* [N, obs_dim] */
+  float* action_bias;       /* [N, action_dim] */
   LgTorchRng* torch_rng;   /* P.rng_stream == LG_RNG_TORCH: the generator state (NULL otherwise)  */
 } LgBuffers;
 

@@ -72,6 +72,8 @@ class LgParams(C.Structure):
         ("max_com_distance", C.c_double),
         ("dr_action_sigma", C.c_float), ("dr_sigma", C.c_float * LG_MAX_STATE_DIM), ("_pad_tail", C.c_int32),
         ("rng_stream", C.c_int32), ("sm_count", C.c_int32), ("threads_per_sm", C.c_int32), ("_pad_tail2", C.c_int32),
+        ("dr_bias_sigma", C.c_float * 64), ("dr_bias_mask", C.c_uint64),
+        ("dr_action_bias_sigma", C.c_float), ("_pad_tail3", C.c_int32),
     ]
 
 
@@ -100,6 +102,7 @@ class LgBuffers(C.Structure):
         "force_reset", "force_goal_reset",
         "episode_return", "last_episode_return", "last_episode_length", "last_episode_success", "episode_stats",
         "episode_term_return", "last_episode_term_return", "episode_term_stats",
+        "obs_bias", "action_bias",
         "torch_rng")]
 
 

@@ -5,7 +5,7 @@ envs/env_base.py:295-309, only writes the config).  A run of this build can stop
 and continue bit-identically: the file holds the goal poses and movement, step counters, reset /
 goal-reset / success flags, the one-deep history, the last action / outputs, the per-step
 statistics (and, with "episode_statistics" on, the running returns and last-episode records; with
-"episode_term_returns" on, their per-term rows too), the device control block (RNG epoch of the kernel's Philox stream, frame counter,
+"episode_term_returns" on, their per-term rows too; with per-episode DR offsets on, each env's offsets), the device control block (RNG epoch of the kernel's Philox stream, frame counter,
 compaction epoch) and the state of the torch CUDA stream (`rng_stream` "torch": seed, offset) — plus, for `SyntheticSim`, the simulator tensors and its clock, because the
 pre-physics pass of the next step reads (and the resets wrote) simulator memory.
 
@@ -20,6 +20,8 @@ from typing import Dict
 
 import numpy as np
 import torch
+
+from .params import dr_bias_sigmas
 
 FORMAT_VERSION = 1
 
@@ -39,6 +41,8 @@ _ENV_TENSORS = {
     # per-term episode returns (absent when that extension is off)
     "episode_term_return": "_episode_term_return", "last_episode_term_return": "_last_episode_term_return",
     "episode_term_stats": "_episode_term_stats",
+    # per-episode DR offsets (each absent when its sigmas are all zero)
+    "obs_bias": "_obs_bias", "action_bias": "_action_bias",
 }
 _SIM_TENSORS = ("dof_state", "root_state", "rigid_body", "dof_force", "ft_sensors")
 
@@ -62,7 +66,8 @@ def env_state_dict(env) -> Dict[str, object]:
         "format": FORMAT_VERSION, "num_instances": int(env.num_instances), "global_num_instances": int(env._global_N),
         "env_offset": int(env._env_offset), "obs_dim": int(env.get_obs_dim()), "state_dim": int(env.get_state_dim()),
         "action_dim": int(env.get_action_dim()), "episode_statistics": _episode_statistics(env.config),
-        "episode_term_returns": _activated(env.config, "episode_term_returns"), "sim": sim_meta, "config": json.loads(json.dumps(env.config, default=str)),
+        "episode_term_returns": _activated(env.config, "episode_term_returns"),
+        "dr_bias": _dr_bias(env.config), "sim": sim_meta, "config": json.loads(json.dumps(env.config, default=str)),
     }
     return out
 
@@ -92,6 +97,11 @@ def load_env_state_dict(env, state: Dict[str, object]) -> None:
     ck_terms = bool(meta.get("episode_term_returns", _activated(meta.get("config", {}), "episode_term_returns")))
     if ck_terms != have_terms:
         raise ValueError(f"checkpoint was written with episode_term_returns.activate={ck_terms}, this env has {have_terms}")
+    have_bias = _dr_bias(env.config)
+    ck_bias = list(meta.get("dr_bias", _dr_bias(meta.get("config", {}))))
+    if ck_bias != have_bias:
+        raise ValueError(f"checkpoint was written with per-episode DR offsets (domain_randomization obs_bias_std / "
+                         f"action_bias_std) on for [obs, action] = {ck_bias}, this env has {have_bias}")
     for name, attr in _ENV_TENSORS.items():
         t = getattr(env, attr, None)
         arr = state.get(f"env/{name}")
@@ -124,6 +134,12 @@ def load_env_state_dict(env, state: Dict[str, object]) -> None:
 
 def _episode_statistics(config: dict) -> bool:
     return _activated(config, "episode_statistics")
+
+
+def _dr_bias(config: dict) -> list:
+    """[obs offsets on, action offsets on]: which offset arrays the env keeps."""
+    obs, act = dr_bias_sigmas(config)
+    return [any(v != 0.0 for v in obs.values()), act != 0.0]
 
 
 def _activated(config: dict, key: str) -> bool:

@@ -102,6 +102,12 @@ def default_trifinger_config() -> Dict[str, Any]:
             # trifinger_env.py:979); the critic's states stay clean
             "obs_noise_std": {"robot_q": 0.0, "robot_u": 0.0, "object_q": 0.0, "object_q_des": 0.0, "command": 0.0},
             "action_noise_std": 0.0,  # additive Gaussian on the action before clipping
+            # per-episode offsets, drawn N(0, sigma^2) per env and column whenever the env is reset (not by a goal-only
+            # reset) and held for the whole episode: a calibration error of the cube pose, an encoder bias, an action
+            # offset.  Added to the raw actor observation before the noise above, and to the action before the noise
+            # and the clip; env.obs_bias / env.action_bias hold them
+            "obs_bias_std": {"robot_q": 0.0, "robot_u": 0.0, "object_q": 0.0, "object_q_des": 0.0, "command": 0.0},
+            "action_bias_std": 0.0,
         },
         # where reset / goal samples come from: "philox" = this build's own counter stream, keyed by (seed, global env
         # id), the same for any sharding; "torch" = the numbers the reference's own torch.rand / torch.randn calls on

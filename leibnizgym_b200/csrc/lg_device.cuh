@@ -210,7 +210,8 @@ __device__ __forceinline__ void box_muller(uint32_t a, uint32_t b, float& n0, fl
   n1 = r * sn;
 }
 
-enum DrawPurpose : uint32_t { kPurposeReset = 0x52455345u, kPurposeGoal = 0x474f414cu, kPurposeNoise = 0x4e4f4953u };
+enum DrawPurpose : uint32_t { kPurposeReset = 0x52455345u, kPurposeGoal = 0x474f414cu, kPurposeNoise = 0x4e4f4953u,
+                              kPurposeBias = 0x42494153u };
 
 // Random numbers of ONE env for ONE reset call.  Either Philox keyed by
 // (seed, global env id, purpose, epoch) or rows of injected arrays (test hook).
@@ -508,6 +509,37 @@ __device__ __noinline__ void end_episode(const LgBuffers& B, int64_t e, int64_t 
     rec[0] = a; rec[1] = b;
     run[0] = run[1] = make_float4(0.f, 0.f, 0.f, 0.f);
   }
+}
+
+// extension (no reference code): the per-episode domain-randomisation offsets of env e, redrawn by its reset.  Always
+// this build's Philox stream keyed by (seed, global env id, kPurposeBias, `epoch` = that of the reset's own draws),
+// whatever stream or injected arrays the reset itself reads.  Philox block b < kBiasActionBlock holds obs columns
+// 4b .. 4b+3 and is drawn only when one of them has sigma != 0; block kBiasActionBlock + b holds action columns
+// 4b .. 4b+3.  Columns with sigma = 0 are stored as +0.0 (sigma x n would be -0.0 for n < 0).  draw_bias_block writes
+// what block `b` covers (nothing for a block beyond the row); draw_bias all of them.
+constexpr int kBiasActionBlock = 16;   // beyond the widest observation (50 columns: blocks 0 .. 12)
+__device__ __forceinline__ void draw_bias_block(const LgParams& P, const LgBuffers& B, int64_t e, uint64_t epoch, int b) {
+  const bool act = b >= kBiasActionBlock;
+  const int width = act ? P.action_dim : 32 + P.action_dim, c0 = 4 * (act ? b - kBiasActionBlock : b);
+  float* row = act ? B.action_bias : B.obs_bias;
+  if (!row || c0 >= width) return;
+  row += e * width;
+  const unsigned m = act ? (P.dr_action_bias_sigma != 0.0f ? 15u : 0u) : (unsigned)(P.dr_bias_mask >> c0) & 15u;
+  float n[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+  if (m) {
+    const U4 r = make_draws(P, epoch, e, kPurposeBias, nullptr, nullptr, 0).block((uint32_t)b);
+    box_muller(r.x, r.y, n[0], n[1]);
+    box_muller(r.z, r.w, n[2], n[3]);
+  }
+#pragma unroll
+  for (int q = 0; q < 4; ++q)
+    if (c0 + q < width)
+      row[c0 + q] = ((m >> q) & 1u) ? (act ? P.dr_action_bias_sigma : P.dr_bias_sigma[c0 + q]) * n[q] : 0.0f;
+}
+// Out of line: the hook kernels keep their registers.
+__device__ __noinline__ void draw_bias(const LgParams& P, const LgBuffers& B, int64_t e, uint64_t epoch) {
+#pragma unroll 1
+  for (int b = 0; b < kBiasActionBlock + (LG_MAX_ACTION_DIM + 3) / 4; ++b) draw_bias_block(P, B, e, epoch, b);
 }
 
 // _reset_impl for ONE env (trifinger_env.py:373-411, :1101-1192) cut into TEN independent sub-tasks, so that the

@@ -10,6 +10,7 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -200,6 +201,22 @@ int validate(const LgParams* P, const LgSimState* S, const LgBuffers* B, bool ne
                                 "last_episode_return, last_episode_length, last_episode_success, episode_stats)");
   if (term_ptrs && (!aligned16(B->episode_term_return) || !aligned16(B->last_episode_term_return)))
     return fail(LG_ERR_BAD_ARG, "episode_term_return and last_episode_term_return must be 16-byte aligned");
+  // per-episode DR offsets: sigmas only on observation columns, the mask marking exactly the nonzero ones
+  uint64_t mask = 0;
+  for (int c = 0; c < 64; ++c) {
+    const float sg = P->dr_bias_sigma[c];
+    if (sg != 0.0f && (c >= 32 + P->action_dim || !std::isfinite(sg) || sg < 0.0f))
+      return fail(LG_ERR_BAD_ARG, "dr_bias_sigma: finite, >= 0, and only on the obs_dim observation columns");
+    if (sg != 0.0f) mask |= 1ull << c;
+  }
+  if (mask != P->dr_bias_mask) return fail(LG_ERR_BAD_ARG, "dr_bias_mask must mark exactly the columns with dr_bias_sigma != 0");
+  if ((mask || P->dr_action_bias_sigma != 0.0f) && !P->dr_activate)
+    return fail(LG_ERR_BAD_ARG, "dr_bias_sigma / dr_action_bias_sigma != 0 need dr_activate");
+  if (mask && !B->obs_bias) return fail(LG_ERR_BAD_ARG, "dr_bias_sigma != 0 needs LgBuffers.obs_bias");
+  const float asg = P->dr_action_bias_sigma;
+  if (asg != 0.0f && (!std::isfinite(asg) || asg < 0.0f))
+    return fail(LG_ERR_BAD_ARG, "dr_action_bias_sigma must be finite and >= 0");
+  if (asg != 0.0f && !B->action_bias) return fail(LG_ERR_BAD_ARG, "dr_action_bias_sigma != 0 needs LgBuffers.action_bias");
   return LG_OK;
 }
 
@@ -389,7 +406,14 @@ cudaError_t err;
   }
 #undef LG_PRE
   if (err != cudaSuccess) return fail(LG_ERR_CUDA, std::string("pre_physics_kernel: ") + cudaGetErrorString(err));
-  return check_launch("pre_physics_kernel");
+  if (int rc = check_launch("pre_physics_kernel")) return rc;
+  if (!B->obs_bias && !B->action_bias) return LG_OK;
+  // extension: the per-episode DR offsets of the envs this pass reset (lg_pre.cuh, draw_bias_kernel): a warp per env
+  const int64_t want = (P->num_envs * 32 + lg::kDrawBiasThreads - 1) / lg::kDrawBiasThreads;
+  const unsigned grid = (unsigned)(want < 8 * sm_count() ? want : 8 * sm_count());
+  err = launch_pdl(pdl_mode() & 2, lg::draw_bias_kernel, grid, lg::kDrawBiasThreads, 0, st, *P, *B);
+  if (err != cudaSuccess) return fail(LG_ERR_CUDA, std::string("draw_bias_kernel: ") + cudaGetErrorString(err));
+  return check_launch("draw_bias_kernel");
 }
 }  // namespace
 
@@ -422,7 +446,11 @@ static int reset_list(const LgParams* P, const LgSimState* S, const LgBuffers* B
     lg::reset_ids_kernel<true><<<(unsigned)((k + 127) / 128), 128, 0, (cudaStream_t)stream>>>(*P, *S, *B, ids, k, goal_only);
     if (int rc = check_launch("reset_ids_kernel")) return rc;
     lg::torch_advance_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(B->torch_rng, lg::torch_plan(*P, (uint32_t)k, goal_only != 0).total());
-    return check_launch("torch_advance_kernel");
+    if (int rc = check_launch("torch_advance_kernel")) return rc;
+    // the DR offsets come from the own stream, keyed by the epoch, also here: each call must draw new ones
+    if (!B->obs_bias && !B->action_bias) return LG_OK;
+    lg::bump_epoch_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(B->control);
+    return check_launch("bump_epoch_kernel");
   }
   lg::reset_ids_kernel<<<(unsigned)((k + 127) / 128), 128, 0, (cudaStream_t)stream>>>(*P, *S, *B, ids, k, goal_only);
   if (int rc = check_launch("reset_ids_kernel")) return rc;
@@ -600,6 +628,8 @@ int lg_step_host_pipelined(const LgParams* P, const LgSimState* S, const LgBuffe
     if (bc.episode_term_return) {
       bc.episode_term_return += lo * LG_NUM_EPISODE_TERMS; bc.last_episode_term_return += lo * LG_NUM_EPISODE_TERMS;
     }
+    if (bc.obs_bias) bc.obs_bias += lo * od;
+    if (bc.action_bias) bc.action_bias += lo * A;
     if (int rc = lg_upload_sim_state(&pc, &sc, &hc, stream_up)) return rc;
     cudaEventRecord(pool.up[c], up);
     cudaStreamWaitEvent(main, pool.up[c], 0);

@@ -51,9 +51,12 @@ __device__ __forceinline__ void bulk_store_commit_and_wait() {
   asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 }
 __device__ __forceinline__ void fence_async_proxy() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-// ---- per-thread asynchronous 16-byte copies (cp.async, SASS LDGSTS): global -> shared without a register ------------
+// ---- per-thread asynchronous 16- and 4-byte copies (cp.async, SASS LDGSTS): global -> shared without a register -----
 __device__ __forceinline__ void async_copy16(void* smem_dst, const void* gmem_src) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" :: "r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
+}
+__device__ __forceinline__ void async_copy4(void* smem_dst, const void* gmem_src) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" :: "r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
 }
 __device__ __forceinline__ void async_copy_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void async_copy_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
@@ -620,6 +623,7 @@ post_physics_kernel(const __grid_constant__ LgParams P, const __grid_constant__ 
   __shared__ float s_part[12][E];       // sub-task results of the reward warps
   __shared__ float s_noise[EXT ? L::OBS : 1][EXT ? E + 1 : 1];   // extension: standard normals of the obs columns
   __shared__ float4 s_term_run[EXT ? 2 * E : 1];   // extension: the tile's running per-term episode returns
+  __shared__ float s_bias[EXT ? L::OBS : 1][EXT ? E + 1 : 1];   // extension: per-episode offsets of the obs columns
 
   const int tid = threadIdx.x;
   const int64_t e0 = (int64_t)blockIdx.x * E;
@@ -690,6 +694,18 @@ post_physics_kernel(const __grid_constant__ LgParams P, const __grid_constant__ 
   } else {
 #pragma unroll
     for (int k = 0; k < EP; ++k) v[k] = k < cnt ? ld_stream1(src + (int64_t)k * stride) : 0.0f;
+  }
+  // extension (per-episode DR offsets): an observation lane whose column carries an offset copies it for its envs into
+  // shared memory with the tile's other loads (lanes hold consecutive columns: coalesced along the row), by cp.async so
+  // that no register waits for it; the same lane reads it back when it emits the column.  Every other lane issues
+  // nothing, and dr_bias_mask == 0 skips it all (dr_activate, in the hot parameter lines, is tested first).
+  const bool biased = EXT && P.dr_activate && P.dr_bias_mask != 0 && front && dcol >= 0 && dcol < L::OBS && ((P.dr_bias_mask >> dcol) & 1);
+  if (biased) {
+    const float* bsrc = B.obs_bias + (e0 + env_first) * L::OBS + dcol;
+#pragma unroll
+    for (int k = 0; k < EP; ++k)
+      if (full || k < cnt) async_copy4(&s_bias[dcol][env_first + k], bsrc + (int64_t)k * L::OBS);
+    async_copy_commit();
   }
   // The flags and the step counter are needed last (by the combine): fetched after the tile's loads.  In front of them
   // the compiler turned the flag bytes into predicates at once — a full round trip in which the combine warp had not
@@ -790,9 +806,12 @@ post_physics_kernel(const __grid_constant__ LgParams P, const __grid_constant__ 
     float* ob = B.obs + e0 * L::OBS + ob_off;                                                // trifinger_env.py:983-987
     float* obc = CLIP ? B.obs_clipped + e0 * L::OBS + ob_off : nullptr;                      // vec_task.py:167
     // extension (no reference code; the TODO at trifinger_env.py:979): additive Gaussian noise on the RAW
-    // actor observation, before scale_transform; the critic's states stay clean.  sigma = 0 -> skipped.
+    // actor observation, before scale_transform; the critic's states stay clean.  sigma = 0 -> skipped.  The env's
+    // per-episode offset (loaded above) comes first: (raw + offset) + sigma n.
     const float sigma = (EXT && P.dr_activate && to_obs) ? __ldg(B.scale_table + 3 * LG_MAX_STATE_DIM + dcol) : 0.0f;
     const bool noisy = EXT && __any_sync(0xffffffffu, sigma != 0.0f);
+    const bool perturbed = noisy || biased;
+    if (EXT && biased) async_copy_wait_all();   // this lane's own offsets have landed
     // optional bf16 copies for the policy / value networks (SURVEY.md 8 f2): of the clipped values when the
     // wrapper's clamp is fused in, else of the scaled values
     uint16_t* stb = (EXT && ASYM && B.states_bf16) ? B.states_bf16 + e0 * L::STATE + st_off : nullptr;
@@ -821,10 +840,13 @@ post_physics_kernel(const __grid_constant__ LgParams P, const __grid_constant__ 
         const float sv = div_by_const(v[k] - centre, half_span, rcp_half, amax);
         float ov = sv;
         // sigma = 0 columns (and non-observation lanes) skip it: their noise row is never generated, and 0 * a stale
-        // inf / NaN left in shared memory by an earlier CTA would be NaN
-        if (noisy && sigma != 0.0f) {
-          const float n0 = s_noise[dcol][env_first + k];   // generated before the barrier, see above
-          ov = div_by_const((v[k] + sigma * n0) - centre, half_span, rcp_half, amax);
+        // inf / NaN left in shared memory by an earlier CTA would be NaN.  Columns without an offset skip the add:
+        // raw + 0.0f would turn -0 into +0.
+        if (perturbed && (biased || sigma != 0.0f)) {
+          float x = v[k];
+          if (biased) x = x + s_bias[dcol][env_first + k];
+          if (noisy && sigma != 0.0f) x = x + sigma * s_noise[dcol][env_first + k];   // generated before the barrier
+          ov = div_by_const(x - centre, half_span, rcp_half, amax);
         }
         if (FULLC || k < cnt) emit_one(k, sv, ov);
       }
@@ -835,8 +857,10 @@ post_physics_kernel(const __grid_constant__ LgParams P, const __grid_constant__ 
           if (FULLC || k < cnt) {
             const float x = P.normalize_obs ? __fdiv_rn(2.0f * (v[k] - c0), span) : v[k];
             float xo = x;
-            if (noisy && sigma != 0.0f) {   // the lane's finite envs keep their noise: bit-identical to the fast path
-              const float vn = v[k] + sigma * s_noise[dcol][env_first + k];
+            if (perturbed && (biased || sigma != 0.0f)) {   // the lane's finite envs keep their noise: bit-identical to the fast path
+              float vn = v[k];
+              if (biased) vn = vn + s_bias[dcol][env_first + k];
+              if (noisy && sigma != 0.0f) vn = vn + sigma * s_noise[dcol][env_first + k];
               xo = P.normalize_obs ? __fdiv_rn(2.0f * (vn - c0), span) : vn;
             }
             emit_one(k, x, xo);

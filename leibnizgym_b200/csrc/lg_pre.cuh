@@ -199,6 +199,18 @@ __device__ __noinline__ void action_noise(const LgParams& P, uint64_t genv, uint
   }
 }
 
+// extension (no reference code): domain randomisation of one env's action row — its per-episode offset (`bias`, the
+// row its last reset drew; null when off), then the Gaussian noise (`noise`).  One call site in the kernel, out of line.
+template <int A>
+__device__ __noinline__ void perturb_action(const LgParams& P, const float* __restrict__ bias, bool noise, uint64_t genv,
+                                            uint32_t epoch, float* act) {
+  if (bias) {
+#pragma unroll
+    for (int c = 0; c < A; ++c) act[c] = act[c] + bias[c];
+  }
+  if (noise) action_noise<A>(P, genv, epoch, act);
+}
+
 // What the first instructions of the kernel need, as the FIRST kernel parameter: kernel parameters sit in the constant
 // bank in a buffer of their own per launch, so every 64-byte line of them costs a constant-cache miss on first use;
 // the slab copies can be issued after one miss instead of four (pointers otherwise spread over LgSimState, LgBuffers,
@@ -214,7 +226,7 @@ struct PreHot {
 
 // One CTA = one tile of 128 envs, two 128-thread groups working on two independent chains:
 //   row group  (warps 0-3, thread = env): the tile's action and joint-state rows arrive as TMA bulk copies; the action
-//              row is clamped (+ noise, extension), zeroed for resetting envs and kept for the torque;
+//              row is clamped (+ offset and noise, extension), zeroed for resetting envs and kept for the torque;
 //   scan group (warps 4-7, thread = env): flag bytes -> ballot/popcount block scan of both masks -> aggregate
 //              published -> block-wide decoupled look-back -> ascending id lists (torch.nonzero order) and the
 //              simulator's actor-index lists.
@@ -437,11 +449,16 @@ pre_physics_kernel(const __grid_constant__ PreHot H, const __grid_constant__ LgP
       const bool zero_row = (s_flag[gt] & 1) != 0;
 #pragma unroll
       for (int c = 0; c < A; ++c) act[c] = s_act[gt * A + c];
-      if (P.dr_activate && P.dr_action_sigma != 0.0f) {   // extension (no reference code): Gaussian action noise
+      // extension (no reference code): per-episode action offset, then Gaussian action noise.  An env that resets in
+      // this step stores 0 below, so its offset row being redrawn by this pass meanwhile does not matter.
+      // dr_activate (hot parameter line) is tested first: the two sigmas sit in cold lines of the parameter block.
+      const bool noise = P.dr_activate && P.dr_action_sigma != 0.0f;
+      if (P.dr_activate && (noise || P.dr_action_bias_sigma != 0.0f)) {
         float noisy[A];                                    // a copy: `act` itself must stay in registers
 #pragma unroll
         for (int c = 0; c < A; ++c) noisy[c] = act[c];
-        action_noise<A>(P, (uint64_t)(P.env_offset + e), epoch, noisy);
+        perturb_action<A>(P, P.dr_action_bias_sigma != 0.0f ? B.action_bias + e * A : nullptr, noise,
+                          (uint64_t)(P.env_offset + e), epoch, noisy);
 #pragma unroll
         for (int c = 0; c < A; ++c) act[c] = noisy[c];
       }
@@ -674,25 +691,42 @@ template <bool TORCH = false>
 __global__ void reset_ids_kernel(const __grid_constant__ LgParams P, const LgSimState S, const LgBuffers B,
                                  const int64_t* __restrict__ ids, int64_t k, int goal_only) {
   const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= k) return;
+  const int64_t e = ids[j];
+  // never collides with the fused path's epochs; keys the own stream's draws and, on either stream, the DR offsets
+  const uint64_t epoch = B.control->rng_epoch | (1ull << 63);
   if constexpr (TORCH) {   // the list's rank j is the env's index in the reference's calls
-    if (j >= k) return;
-    const int64_t e = ids[j];
     const TorchDraws dr = make_torch_draws(P, B.torch_rng->seed, B.torch_rng->offset, (uint32_t)k, goal_only != 0, j);
     if (goal_only) hook_goal_env(P, S, B, e, j, dr);
     else hook_reset_env(P, S, B, e, j, dr);
-  } else if (j < k) {
-    const int64_t e = ids[j];
-    const uint64_t epoch = B.control->rng_epoch | (1ull << 63);  // never collides with the fused path's epochs
+    if (!goal_only && (B.obs_bias || B.action_bias)) draw_bias(P, B, e, epoch);   // extension: new offsets
+  } else {
     if (goal_only) {
       const DrawSource dr = make_draws(P, epoch, e, kPurposeGoal, B.inject_goal_u, B.inject_goal_n, j);
       hook_goal_env(P, S, B, e, j, dr);
     } else {
       const DrawSource dr = make_draws(P, epoch, e, kPurposeReset, B.inject_reset_u, B.inject_reset_n, j);
       hook_reset_env(P, S, B, e, j, dr);
+      if (B.obs_bias || B.action_bias) draw_bias(P, B, e, epoch);
     }
   }
 }
 __global__ void bump_epoch_kernel(LgControl* ctl) { ctl->rng_epoch += 1; }
+
+// extension (per-episode DR offsets): the envs the pre-physics launch in front of it reset (its reset list) draw their
+// new offsets, keyed like that launch's own draws by the compaction epoch it ran under (it advanced scan_epoch by one on
+// its way out).  One warp per listed env, lane = Philox block (draw_bias_block), grid-stride over the list.  A launch of
+// its own, made only when the offsets are on: inside the pre-physics pass the draw cost every one of its instantiations
+// spills, whether the offsets were on or not.  Launched programmatically: it becomes resident while that pass finishes.
+constexpr int kDrawBiasThreads = 256;
+__global__ void __launch_bounds__(kDrawBiasThreads) draw_bias_kernel(const __grid_constant__ LgParams P, const LgBuffers B) {
+  pdl_launch_dependents();   // the post-physics pass may become resident; it waits for this grid to complete
+  pdl_wait();                // the reset list and the epoch are results of the pre-physics pass
+  const int64_t n = (int64_t)B.counts[0] * 32;
+  const uint64_t epoch = (uint32_t)(ld_volatile_u32(&B.control->scan_epoch) - 1u);
+  for (int64_t t = (int64_t)blockIdx.x * kDrawBiasThreads + threadIdx.x; t < n; t += (int64_t)gridDim.x * kDrawBiasThreads)
+    draw_bias_block(P, B, B.reset_ids[t >> 5], epoch, (int)(t & 31));
+}
 
 __global__ void pre_step_kernel(const __grid_constant__ LgParams P, const LgSimState S, const LgBuffers B) {
   const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;

@@ -27,7 +27,7 @@ import yaml
 
 from . import _native as nat
 from .config import resolve_config
-from .params import action_dim_of, action_scale, build_params, observation_scale, state_scale
+from .params import action_dim_of, action_scale, build_params, dr_bias_sigmas, observation_scale, state_scale
 from .sim import LazyCount, SyntheticSim
 from .synthetic import make_sequence
 
@@ -175,11 +175,13 @@ class IsaacEnvBase:
         """Generic hook-by-hook sequencing (ref env_base.py:345-401); TrifingerEnv overrides it
         with the fused two-launch version."""
         dr = self.config.get("domain_randomization") or {}
-        if dr.get("activate") and float(dr.get("action_noise_std", 0.0)) != 0.0:
-            # the action noise is keyed by the compaction epoch, which only the fused pre-physics pass advances: hook
-            # steps would store the raw action and, if they drew at all, draw the same noise every step
-            raise ValueError("domain_randomization.action_noise_std > 0 is applied by the fused step only: "
-                             "step with TrifingerEnv.step, not the hook-by-hook IsaacEnvBase.step")
+        for key in ("action_noise_std", "action_bias_std"):
+            if dr.get("activate") and float(dr.get(key, 0.0)) != 0.0:
+                # the action noise is keyed by the compaction epoch, which only the fused pre-physics pass advances:
+                # hook steps would store the raw action and, if they drew at all, draw the same noise every step.  The
+                # action offset is added by that pass too
+                raise ValueError(f"domain_randomization.{key} > 0 is applied by the fused step only: "
+                                 "step with TrifingerEnv.step, not the hook-by-hook IsaacEnvBase.step")
         self._step_info = {}
         action = self._check_action(action)
         self._action_buf.copy_(action)
@@ -265,6 +267,7 @@ class TrifingerEnv(IsaacEnvBase):
         if cfg["episode_term_returns"]["activate"] and not cfg["episode_statistics"]["activate"]:
             raise ValueError('"episode_term_returns" needs "episode_statistics": {"activate": True}: the per-term '
                              "returns are kept and reported with the episode statistics")
+        dr_bias_sigmas(cfg)   # a bad sigma or group of the per-episode DR offsets raises here, before any device work
         obs_spec = {"robot_q": 9, "robot_u": 9, "object_q": 7, "object_q_des": 7, "command": A}
         if cfg["asymmetric_obs"]:
             state_spec = dict(obs_spec, object_u=6, fingertip_state=39, robot_a=9, fingertip_wrench=18)
@@ -326,6 +329,12 @@ class TrifingerEnv(IsaacEnvBase):
             self._episode_term_return = torch.zeros((N, T), device=dev, dtype=torch.float)
             self._last_episode_term_return = torch.zeros((N, T), device=dev, dtype=torch.float)
             self._episode_term_stats = torch.zeros(T, device=dev, dtype=torch.float64)
+        # extension: per-episode DR offsets, each allocated only when one of its sigmas is nonzero
+        obs_sig, act_sig = dr_bias_sigmas(self.config)
+        A = action_dim_of(self.config["command_mode"])
+        self._obs_bias = (torch.zeros((N, 32 + A), device=dev, dtype=torch.float)
+                          if any(v != 0.0 for v in obs_sig.values()) else None)
+        self._action_bias = torch.zeros((N, A), device=dev, dtype=torch.float) if act_sig != 0.0 else None
         self._reset_ids = torch.zeros(N, device=dev, dtype=torch.long)
         self._goal_reset_ids = torch.zeros(N, device=dev, dtype=torch.long)
         self._counts = torch.zeros(2, **i32)
@@ -396,6 +405,7 @@ class TrifingerEnv(IsaacEnvBase):
         b.episode_stats = p(self._episode_stats)
         b.episode_term_return, b.last_episode_term_return = p(self._episode_term_return), p(self._last_episode_term_return)
         b.episode_term_stats = p(self._episode_term_stats)
+        b.obs_bias, b.action_bias = p(self._obs_bias), p(self._action_bias)
         self._B = b
         if not getattr(self, "_history_seeded", False):
             self._call("lg_init_history", self._P, self._S, self._B)  # ref trifinger_env.py:619-628
@@ -635,6 +645,22 @@ class TrifingerEnv(IsaacEnvBase):
         if self.config["termination_conditions"]["success"]["activate"]:
             names.append("success_bonus")
         return names
+
+    # -- per-episode DR offsets (extension, "domain_randomization": obs_bias_std / action_bias_std; None when off) --
+    # Every reset of an env but a goal-only one (a timeout, a flag or forced mask, `reset()`, `_reset_impl`) draws its
+    # rows anew: sigma x N(0, 1) per column from this build's Philox stream, whatever "rng_stream" says, and 0 where
+    # sigma is 0.  An env never reset holds zeros; `reset()` draws every row.  The actor observation sees
+    # scale_transform((raw + obs_bias) + noise); states, rewards and statistics see the clean values.  The stored
+    # action is clamp((action + action_bias) + noise).
+    @property
+    def obs_bias(self) -> Optional[torch.Tensor]:
+        """[N, obs_dim] fp32: each env's offset of the raw observation columns for its running episode."""
+        return self._obs_bias
+
+    @property
+    def action_bias(self) -> Optional[torch.Tensor]:
+        """[N, action_dim] fp32: each env's offset of the (normalised) action for its running episode."""
+        return self._action_bias
 
     # -- checkpoint / resume (SURVEY.md §8 f4; the reference only dumps its config, env_base.py:295-309) ------
     def state_dict(self) -> dict:

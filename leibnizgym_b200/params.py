@@ -116,6 +116,42 @@ def _fill_terms(p: nat.LgParams, cfg_terms: dict) -> None:
             raise ValueError("finger_reach_object_rate.norm_p: only the 2-norm is built")
 
 
+OBS_GROUPS = ("robot_q", "robot_u", "object_q", "object_q_des", "command")
+
+
+def obs_group_columns(action_dim: int) -> Dict[str, Tuple[int, int]]:
+    """Raw actor observation columns [a, b) of each obs_spec group (trifinger_env.py:280-286)."""
+    return {"robot_q": (0, 9), "robot_u": (9, 18), "object_q": (18, 25), "object_q_des": (25, 32),
+            "command": (32, 32 + action_dim)}
+
+
+def _sigma(value, key: str) -> float:
+    try:
+        s = float(value)
+    except (TypeError, ValueError):
+        raise ValueError(f"{key} must be a number, got {value!r}") from None
+    if not math.isfinite(s) or s < 0.0:
+        raise ValueError(f"{key} must be finite and >= 0, got {value!r}")
+    return s
+
+
+def dr_bias_sigmas(cfg: dict) -> Tuple[Dict[str, float], float]:
+    """Per-episode offsets of "domain_randomization" (extension): (sigma per obs group, sigma of the action offset),
+    all zero unless `activate`.  Raises ValueError naming the key for a negative or non-finite sigma or an unknown
+    group."""
+    dr = cfg.get("domain_randomization") or {}
+    groups = {name: 0.0 for name in OBS_GROUPS}
+    if not dr.get("activate", False):
+        return groups, 0.0
+    obs = dr.get("obs_bias_std") or {}
+    for name, value in obs.items():
+        if name not in groups:
+            raise ValueError(f"domain_randomization.obs_bias_std: unknown observation group {name!r} "
+                             f"(groups: {list(OBS_GROUPS)})")
+        groups[name] = _sigma(value, f"domain_randomization.obs_bias_std.{name}")
+    return groups, _sigma(dr.get("action_bias_std", 0.0), "domain_randomization.action_bias_std")
+
+
 def build_params(cfg: dict, num_local_envs: int, env_offset: int = 0, global_num_envs: int | None = None,
                  fingertip_bodies=(6, 11, 16), bodies_per_env: int = 20, actors_per_env: int = 4,
                  slots=(0, 2, 3), sm_count: int = 0, threads_per_sm: int = 0) -> nat.LgParams:
@@ -195,11 +231,15 @@ def build_params(cfg: dict, num_local_envs: int, env_offset: int = 0, global_num
     p.dr_action_sigma = float(dr.get("action_noise_std", 0.0)) if p.dr_activate else 0.0
     if p.dr_activate:  # sigma per RAW observation column, by the obs_spec groups (trifinger_env.py:280-286)
         std = dr.get("obs_noise_std", {})
-        groups = (("robot_q", 0, 9), ("robot_u", 9, 18), ("object_q", 18, 25), ("object_q_des", 25, 32),
-                  ("command", 32, 32 + A))
-        for name, a, b in groups:
+        for name, (a, b) in obs_group_columns(A).items():
             for c in range(a, b):
                 p.dr_sigma[c] = float(std.get(name, 0.0))
+    obs_bias, p.dr_action_bias_sigma = dr_bias_sigmas(cfg)   # per-episode offsets (zero unless activate)
+    for name, (a, b) in obs_group_columns(A).items():
+        for c in range(a, b):
+            p.dr_bias_sigma[c] = obs_bias[name]
+            if p.dr_bias_sigma[c] != 0.0:
+                p.dr_bias_mask |= 1 << c
     p.seed = int(cfg["seed"]) & 0xFFFFFFFFFFFFFFFF
     p.rng_stream = nat.RNG_STREAMS[stream]
     p.sm_count, p.threads_per_sm = int(sm_count), int(threads_per_sm)
