@@ -9,6 +9,8 @@ from __future__ import annotations
 import numpy as np
 import torch
 
+from .trifinger_oracle import OracleEnv, scale_transform
+
 CUBE_SIZE = 0.065
 
 
@@ -56,3 +58,28 @@ def integrate_goal_rows(rows: np.ndarray, dt: float) -> np.ndarray:
     r[:, 3:7] = out / np.linalg.norm(out, axis=1, keepdims=True)
     r[:, 0:3] += r[:, 7:10] * dt
     return r
+
+
+class OffsetOracleEnv(OracleEnv):
+    """OracleEnv whose actor observation carries per-episode DR offsets (extension "domain_randomization":
+    obs_bias_std): obs = scale_transform(raw + obs_bias) on the columns `bias_cols` (those with sigma != 0; the others
+    keep their raw value, -0 included); states stay clean.  The caller sets `obs_bias` [N, obs_dim] to the rows the
+    env's resets drew and steps with the perturbed action (action + action offset, clamped like the env)."""
+
+    obs_bias = None
+    bias_cols = ()
+
+    def fill_observations_and_states(self):
+        norm = self.cfg["normalize_obs"]
+        self.cfg["normalize_obs"] = False
+        try:
+            super().fill_observations_and_states()
+        finally:
+            self.cfg["normalize_obs"] = norm
+        if self.obs_bias is not None and len(self.bias_cols):
+            c = list(self.bias_cols)
+            self.obs_buf[:, c] = self.obs_buf[:, c] + self.obs_bias[:, c]
+        if norm:
+            self.obs_buf = scale_transform(self.obs_buf, self.obs_lo, self.obs_hi)
+            if self.asym:
+                self.states_buf = scale_transform(self.states_buf, self.st_lo, self.st_hi)

@@ -5,17 +5,18 @@
 
 The launcher's switches (LG_TILE_ENVS, LG_PRE_TICKET, LG_PRE_DIRECT, LG_PDL) are read once per process, so every forced
 setting runs in a process of its own and prints one JSON line per scenario: a sha256 per buffer group, the episode
-statistics, and the instantiations of the two fused kernels that ran (`launched`, parsed from torch.profiler).
+statistics (step and episode), and the instantiations of the two fused kernels that ran (`launched`, parsed from torch.profiler).
 
-Scenario "ext:<a|s>:<A>:<N>:<own|torch>:<route>": difficulty 4 with DR observation and action noise, the keypoint term,
-the moving goal (integrated by the synthetic simulator), bf16 copies, the wrapper's fused clamps, success termination,
-30 % forced resets and 5 % forced goal resets, 4 steps after reset().  Routes:
+Scenario "ext:<a|s>:<A>:<N>:<own|torch>:<route>": difficulty 4 with DR observation and action noise, per-episode DR
+observation and action offsets, the keypoint term, the moving goal (integrated by the synthetic simulator), bf16
+copies, the wrapper's fused clamps, success termination, episode statistics and per-term episode returns, 30 % forced
+resets and 5 % forced goal resets, 4 steps after reset().  Routes:
   eager   VecTaskPython.step
   graph   GraphRunner with the device clock, captured and replayed (clamps off: the runner's buffers have none; env
           counts divisible by 4, so that every output slot is 16-byte aligned, and still ragged at every tile size)
   host    GraphRunner with the host clock, stepped eagerly through the same sequence as `graph`
   shards  two shards of N / 2 envs (world_size 2), outputs concatenated: equal to `eager` except ids and statistics
-  fused / hooks   TrifingerEnv.step against IsaacEnvBase.step: no clamps and no action noise (the hook route refuses it)
+  fused / hooks   TrifingerEnv.step against IsaacEnvBase.step: no clamps, no action noise and no DR offsets (see config)
 """
 import copy
 import hashlib
@@ -31,6 +32,7 @@ sys.path.insert(0, ROOT)
 
 T = 4
 SIGMA = {"robot_q": 0.01, "robot_u": 0.05, "object_q": 0.002, "object_q_des": 0.001, "command": 0.01}
+BIAS = {"robot_q": 0.02, "robot_u": 0.1, "object_q": 0.005, "object_q_des": 0.003, "command": 0.03}
 SUCCESS = {"success": {"activate": True, "bonus": 500.0, "position_tolerance": 0.05, "orientation_tolerance": 1.0}}
 DEFAULT = ["ext:a:9:12343:own:eager", "ext:s:9:12343:own:eager", "ext:a:9:16381:own:eager", "ext:s:9:16381:own:eager",
            "ext:a:9:16384:own:eager", "ext:a:18:12343:own:eager", "ext:s:18:16381:own:eager",
@@ -68,6 +70,8 @@ def launched(fn):
 
 
 def config(N, asym, A, stream, action_noise=True):
+    """`action_noise=False`: no action noise and no DR offsets, for the hook route.  It refuses the action noise and
+    the action offsets, and its resets key their draws by an epoch of their own, so its offset rows differ."""
     from leibnizgym_b200.config import difficulty_config
     cfg = difficulty_config(4, N, asymmetric_obs=asym, seed=23, episode_length=3,
                             command_mode="torque" if A == 9 else "position_impedance",
@@ -75,7 +79,10 @@ def config(N, asym, A, stream, action_noise=True):
                             goal_movement={"rotation": {"activate": True, "rate_magnitude": 0.5}})
     cfg["reward_terms"]["keypoint"] = {"activate": True, "weight": 1500, "scale": 30.0, "eps": 2.0}
     cfg["domain_randomization"] = {"activate": True, "action_noise_std": 0.03 if action_noise else 0.0,
-                                   "obs_noise_std": dict(SIGMA)}
+                                   "obs_noise_std": dict(SIGMA), "obs_bias_std": dict(BIAS) if action_noise else {},
+                                   "action_bias_std": 0.05 if action_noise else 0.0}
+    cfg["episode_statistics"] = {"activate": True}
+    cfg["episode_term_returns"] = {"activate": True}
     cfg["rng_stream"] = "philox" if stream == "own" else stream
     return cfg
 
@@ -107,8 +114,16 @@ def groups(envs, obs=None, states=None):
                     torch.cat([e._sim.root_state.reshape(e.num_instances, -1) for e in envs])),
         "ids": _sha(*[torch.cat([e._reset_ids[: int(e._counts[0])], e._goal_reset_ids[: int(e._counts[1])]])
                       for e in envs]),
+        "episodes": _sha(cat("_episode_return"), cat("_last_episode_return"), cat("_last_episode_length"),
+                         cat("_last_episode_success"), cat("_episode_term_return"), cat("_last_episode_term_return")),
+        "offsets": _sha(cat("_obs_bias"), cat("_action_bias")),
     }
     return out
+
+
+def episode_stats(env):
+    """The step's `_episode_stats` and `_episode_term_stats` (fp64 sums of the CTAs' fixed-point parts)."""
+    return env._episode_stats.tolist() + env._episode_term_stats.tolist()
 
 
 def run(name):
@@ -152,7 +167,7 @@ def run(name):
             runner.t, runner.t0 = 0, -2
             runner.step_eager(T)
         torch.cuda.synchronize()
-        return groups([env], runner.obs_slots, runner.state_slots), env._step_stats.tolist(), kernels
+        return groups([env], runner.obs_slots, runner.state_slots), env._step_stats.tolist(), episode_stats(env), kernels
 
     world = 2 if route == "shards" else 1
     n = N // world
@@ -187,13 +202,14 @@ def run(name):
                 step()
     torch.cuda.synchronize()
     stats = [e._step_stats.tolist() for e in envs]
-    return groups(envs), stats[0] if world == 1 else stats, kernels
+    episodes = [episode_stats(e) for e in envs]
+    return groups(envs), stats[0] if world == 1 else stats, episodes[0] if world == 1 else episodes, kernels
 
 
 def main(argv):
     for name in argv or DEFAULT:
-        digests, stats, kernels = run(name)
-        print(json.dumps({"scenario": name, "digests": digests, "stats": stats,
+        digests, stats, episodes, kernels = run(name)
+        print(json.dumps({"scenario": name, "digests": digests, "stats": stats, "episode_stats": episodes,
                           "launched": {k: sorted(v) for k, v in kernels.items()}}), flush=True)
 
 

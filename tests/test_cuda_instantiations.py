@@ -3,13 +3,14 @@ launch_post, launch_pre), each tested where it is picked, and each case checked 
 
   a. which kernel ran: torch.profiler names the instantiation; the coverage test matches the library's own symbol
      table against the instantiations the cases below claim;
-  b. oracle parity at the launcher's own choice, for every post-physics tile size with ragged tiles of
+  b. oracle parity (tests/lockstep.py: every output, every step) at the launcher's own choice, for every post-physics tile size with ragged tiles of
      nvalid in {1, EP - 1, EP, EP + 1, E - 1} envs (EP = envs per role-lane part), every pre-physics grid regime,
      action_dim 9 and 18; the torch stream's fused step against its hook-by-hook step in every pre-physics regime;
   c. bit-exact invariance with every extension on across forced tile sizes, forced pre-physics paths, PDL off, two
      shards split inside a noise group, graph replay with the device clock, and the hook-by-hook route
      (tests/instantiation_digest.py, one process per forced setting);
-  d. DR observation noise next to a diverged env: the lane's other envs keep their noisy observations bit for bit.
+  d. DR observation noise and offsets next to a diverged env: the lane's other envs keep their perturbed observations
+     bit for bit, and the diverged env's IEEE redo keeps its offset.
 """
 import copy
 import json
@@ -25,8 +26,8 @@ import torch
 
 from instantiation_digest import DEFAULT as DIGEST_SCENARIOS
 from instantiation_digest import kernel_args, launched
-from test_cuda_edges import SUCCESS, _angle_allowance, _check, _check_info, _np, _tile_envs
-from tolerances import compare
+from lockstep import Lockstep, rf_same
+from test_cuda_edges import SUCCESS, _np, _tile_envs
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
@@ -138,143 +139,19 @@ def test_every_built_instantiation_is_claimed_by_a_case():
 
 
 # ======== b. oracle parity per geometry ===================================================================================
-class _Run:
-    """A CUDA env (through VecTaskPython when the clamps are fused in) and the oracle in lockstep, with injected draws,
-    30 % forced resets and 5 % forced goal resets.  ext: keypoint term, moving goal (integrated on both sides), bf16."""
-
-    def __init__(self, A, N, asym, clip, ext, seed):
-        from leibnizgym_b200.config import difficulty_config, resolve_config
-        from leibnizgym_b200.env import TrifingerEnv
-        from leibnizgym_b200.sim import SyntheticSim
-        from leibnizgym_b200.synthetic import bernoulli_masks, make_sequence
-        from leibnizgym_b200.wrappers import VecTaskPython
-        from oracle.extensions import integrate_goal_rows
-        from oracle.trifinger_oracle import OracleEnv, OracleSim
-        self.N, self.T, self.clip, self.ext = N, 5, clip, ext
-        extra = {"goal_movement": {"rotation": {"activate": True, "rate_magnitude": 0.5}}} if ext else {}
-        cfg = difficulty_config(4, N, asymmetric_obs=asym, seed=seed % 97, episode_length=3,
-                                command_mode="torque" if A == 9 else "position_impedance",
-                                termination_conditions=copy.deepcopy(SUCCESS), **extra)
-        ora_cfg = copy.deepcopy(cfg)
-        if ext:
-            cfg["reward_terms"]["keypoint"] = {"activate": True, "weight": 1500, "scale": 30.0, "eps": 2.0}
-        self.seq = make_sequence(seed, self.T, N, action_dim=A)
-        self.masks = bernoulli_masks(seed + 1, self.T, N, 0.3)
-        self.gmasks = bernoulli_masks(seed + 2, self.T, N, 0.05)
-        sim = SyntheticSim(self.seq.to("cuda:0"), "cuda:0")
-        self.env = env = TrifingerEnv(cfg, device="cuda:0", verbose=False, sim=sim)
-        env.enable_term_rewards(True)
-
-        class IntegratingOracleSim(OracleSim):
-            def simulate(self):
-                keep = self.root.view(N, 4, 13)[:, 3].clone()
-                super().simulate()
-                self.root.view(N, 4, 13)[:, 3] = torch.from_numpy(integrate_goal_rows(keep.numpy(), 0.02).astype(np.float32))
-
-        if ext:
-            sim.enable_goal_integration(env._P, 0.02)
-        self.ora = OracleEnv(resolve_config(ora_cfg), (IntegratingOracleSim if ext else OracleSim)(self.seq, N))
-        # the goal pose the rewards see: the moving goal's update (after the termination check) replaces it
-        check_termination = self.ora._check_termination
-
-        def snapshot():
-            self.goal_rewarded = self.ora.goal_poses.clone()
-            check_termination()
-        self.ora._check_termination = snapshot
-        self.vec = None
-        if clip:
-            self.vec = VecTaskPython(env, rl_device="cuda:0", clip_obs=5.0, clip_actions=1.0,
-                                     obs_dtype=torch.bfloat16 if ext else torch.float32)
-        elif ext:
-            env.enable_bf16_outputs()
-        self.g = torch.Generator().manual_seed(seed)
-
-    def _draws(self, k):
-        return (torch.rand(k, 24, generator=self.g).numpy(), torch.randn(k, 8, generator=self.g).numpy()) if k else None
-
-    def reset(self):
-        d = self._draws(self.N)
-        self.env.inject_draws(reset=d)
-        self.ora.inject_draws(reset=d)
-        (self.vec.reset if self.vec is not None else self.env.reset)()
-        self.ora.reset()
-
-    def step(self, t):
-        env, ora = self.env, self.ora
-        ora.reset_buf |= self.masks[t]
-        ora.goal_reset_buf |= self.gmasks[t]
-        env.set_forced_resets(self.masks[t].cuda(), self.gmasks[t].cuda())
-        dr, dg = self._draws(int(ora.reset_buf.sum())), self._draws(int(ora.goal_reset_buf.sum()))
-        env.inject_draws(reset=dr, goal=dg)
-        ora.inject_draws(reset=dr, goal=dg)
-        act = self.seq.action[t]
-        if self.vec is not None:
-            self.vec.step(act.cuda())
-            ora.step(torch.clamp(act, -1.0, 1.0))
-        else:
-            env.step(act.cuda())
-            ora.step(act.clone())
-        return dr is not None, dg is not None
-
-    def check(self, t, reset, goal_reset, where):
-        from oracle.extensions import keypoint_reward
-        env, ora, N = self.env, self.ora, self.N
-        w = where + (t,)
-        torch.cuda.synchronize()
-        # bit-exact: ids, actor-index lists, flags, counters, reset joint rows
-        _check("reset_ids", env.reset_env_ids, ora.last_ids[0], w)
-        _check("goal_reset_ids", env.goal_reset_env_ids, ora.last_ids[1], w)
-        k, kg = int(env._counts[0]), int(env._counts[1])
-        if reset:
-            _check("dof_index_list", env._robot_indices[:k], ora.index_lists["dof"], w)
-            _check("root_index_list0", env._reset_root_indices[:3 * k], ora.index_lists["root_reset"], w)
-        if goal_reset:
-            _check("root_index_list1", env._goal_root_indices[:kg], ora.index_lists["root_goal"], w)
-        for key, got, exp in (("reset_buf", env._reset_buf, ora.reset_buf), ("goal_reset_buf", env._goal_reset_buf,
-                              ora.goal_reset_buf), ("successes", env._successes, ora.successes),
-                              ("steps_count", env._steps_count_buf, ora.steps_count_buf)):
-            _check(key, got, exp, w)
-        assert np.array_equal(_np(env._dof_state).reshape(N, 18), ora.sim.dof.numpy().reshape(N, 18)), (w, "joint rows")
-        # within the tolerances: outputs, action row, torque, terms, reward
-        drift = 2e-6 if self.ext else None       # the moving goal: fp32 integrator against the fp64 oracle
-        _check("goal_pose", env._object_goal_poses_buf, ora.goal_poses, w, drift)
-        _check("goal_movement", env._object_goal_movement_buf, ora.goal_movement, w)
-        clip = lambda x: torch.clamp(x, -5.0, 5.0)  # noqa: E731
-        outs = [("obs", env.obs_buf, ora.obs_buf, env._obs_clipped, env._obs_bf16)]
-        if env.config["asymmetric_obs"]:
-            outs.append(("states", env.states_buf, ora.states_buf, env._states_clipped, env._states_bf16))
-        for key, raw, want, clipped, bf16 in outs:
-            _check(key, raw, want, w, drift)
-            if self.clip:
-                _check(key, clipped, clip(want), w + ("clipped",), drift)
-            if bf16 is not None:
-                src = clipped if self.clip else raw
-                assert torch.equal(bf16.view(torch.int16), src.to(torch.bfloat16).view(torch.int16)), (w, key, "bf16")
-        assert rf_same(env.action_buf, ora.action_buf), (w, "action_buf")
-        _check("applied_torque", env._applied_torque, ora.applied_torque, w)
-        slack_terms, slack_reward = _angle_allowance(ora)
-        if self.ext:   # goal quaternions up to 2e-6 apart (drift above): ~17x the 2 ulp of |v| the allowance assumes
-            slack_terms, slack_reward = 20 * slack_terms, 20 * slack_reward
-        _check("terms", env._term_rewards[:6], ora.last_terms, w, slack_terms)
-        want = ora.reward_buf
-        if self.ext:
-            kp = keypoint_reward(1500, 0.02, ora.obj_hist[0][:, 0:7], self.goal_rewarded)
-            ok, detail = compare("terms", _np(env._term_rewards[6]), kp.numpy(), extra_atol=2e-5 * np.abs(kp.numpy()))
-            assert ok, (w, "keypoint", detail)
-            want = want + kp
-            slack_reward = slack_reward + 5e-4
-        _check("reward", env.reward_buf, want, w, slack_reward)
-        _check_info(env._step_info, ora.step_info, w)
-
-
-def rf_same(a, b):
-    a, b = _np(a), _np(b)
-    return a.shape == b.shape and bool(np.all((a == b) | (np.isnan(a) & np.isnan(b))))
-
-
 def _lockstep(A, N, asym, clip, ext, post_E, pre, where):
-    """Reset + 4 steps against the oracle; reset() and the first step run under the profiler."""
-    run = _Run(A, N, asym, clip, ext, seed=N % 1000 + 7 * A)
+    """Reset + 4 steps against the oracle (tests/lockstep.py) with 30 % forced resets and 5 % forced goal resets;
+    ext: keypoint term, moving goal (integrated on both sides), bf16.  reset() and the first step run under the
+    profiler."""
+    from leibnizgym_b200.config import difficulty_config
+    from leibnizgym_b200.synthetic import bernoulli_masks, make_sequence
+    seed, T = N % 1000 + 7 * A, 5
+    extra = {"goal_movement": {"rotation": {"activate": True, "rate_magnitude": 0.5}}} if ext else {}
+    cfg = difficulty_config(4, N, asymmetric_obs=asym, seed=seed % 97, episode_length=3,
+                            command_mode="torque" if A == 9 else "position_impedance",
+                            termination_conditions=copy.deepcopy(SUCCESS), **extra)
+    run = Lockstep(cfg, make_sequence(seed, T, N, action_dim=A), bernoulli_masks(seed + 1, T, N, 0.3),
+                   bernoulli_masks(seed + 2, T, N, 0.05), seed, clip=clip, bf16=ext, keypoint=ext, goal_integration=ext)
     got = launched(run.reset)
     flags = {}
     got1 = launched(lambda: flags.update(r=run.step(1)))
@@ -283,7 +160,7 @@ def _lockstep(A, N, asym, clip, ext, post_E, pre, where):
     post = {(A, int(asym), r, int(clip), post_E, int(ext)) for r in (0, 1)}
     _expect(got, post=post, pre={(A, *PRE[pre], 0)}, where=where)
     run.check(1, *flags["r"], where)
-    for t in range(2, run.T):
+    for t in range(2, T):
         run.check(t, *run.step(t), where)
 
 
@@ -385,16 +262,28 @@ def _same_stats(a, b, n, where):
         assert np.all(np.abs(a - b) <= 2.0 ** -30 + 1e-12 * np.abs(b)), (where, a, b)
 
 
+def _same_episode_stats(a, b, where):
+    """`_episode_stats` + `_episode_term_stats`: the count, length sum and success count exact; the return sums, whose
+    CTA partition differs between forced tile sizes, to the fixed-point resolution per record."""
+    a, b = np.asarray(a, np.float64), np.asarray(b, np.float64)
+    exact = [0, 2, 3]
+    assert np.array_equal(a[exact], b[exact]), (where, a, b)
+    rest = [i for i in range(len(b)) if i not in exact]
+    assert np.all(np.abs(a[rest] - b[rest]) <= 2.0 ** -30 * b[0] + 1e-12 * np.abs(b[rest])), (where, a, b)
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("setting", SETTINGS, ids=[",".join(f"{k}={v}" for k, v in s.items()) for s in SETTINGS])
 def test_forced_launch_paths_are_bit_identical(default_digests, setting):
     """Each forced tile size / pre-physics path / PDL off, own and torch stream, eager and graph replay: every buffer
-    group equal to the launcher's own choice; the forced instantiation is the one that ran."""
+    group (episode buffers and DR offset rows included) equal to the launcher's own choice; the forced instantiation
+    is the one that ran."""
     forced = _digest_run(setting, FORCED_SCENARIOS)
     for name in FORCED_SCENARIOS:
         got, ref = forced[name], default_digests[name]
         assert got["digests"] == ref["digests"], (setting, name, got["digests"], ref["digests"])
         _same_stats(got["stats"], ref["stats"], int(name.split(":")[3]), (setting, name))
+        _same_episode_stats(got["episode_stats"], ref["episode_stats"], (setting, name))
         post, pre = got["launched"]["post"], got["launched"]["pre"]
         if name.endswith(":graph"):
             continue
@@ -423,6 +312,7 @@ def test_graph_shard_and_route_equivalence(default_digests):
         g, h = d[a + ":graph"], d[a + ":host"]
         assert g["digests"] == h["digests"], (a, g["digests"], h["digests"])
         _same_stats(g["stats"], h["stats"], int(a.split(":")[3]), a)
+        _same_episode_stats(g["episode_stats"], h["episode_stats"], a)
     drop = lambda x, keys: {k: v for k, v in x.items() if k not in keys}  # noqa: E731
     one, two = d["ext:a:9:8198:own:eager"]["digests"], d["ext:a:9:8198:own:shards"]["digests"]
     assert drop(one, ("ids",)) == drop(two, ("ids",)), (one, two)
@@ -451,15 +341,22 @@ def test_hook_route_refuses_action_noise():
     IsaacEnvBase.step(quiet, seq.action[1].cuda())
 
 
-# ======== d. DR observation noise next to a diverged env ==================================================================
+# ======== d. DR observation noise and offsets next to a diverged env =====================================================
+NEIGHBOUR_CASES = [(True, 28, 20, "noise"), (False, 16, 7, "noise"), (True, 28, 20, "offset"), (False, 16, 7, "offset"),
+                   (True, 28, 20, "both"), (False, 16, 7, "both")]
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("value", [2.0 ** 100, float("inf"), float("nan")], ids=["2^100", "inf", "nan"])
-@pytest.mark.parametrize("asym, E, last", [(True, 28, 20), (False, 16, 7)], ids=["a-E28", "s-E16"])
-def test_noisy_neighbours_of_a_diverged_env_are_unchanged(value, asym, E, last):
+@pytest.mark.parametrize("asym, E, last, perturb", NEIGHBOUR_CASES,
+                         ids=[f"{'a' if c[0] else 's'}-E{c[1]}" + ("" if c[3] == "noise" else f"-{c[3]}")
+                              for c in NEIGHBOUR_CASES])
+def test_noisy_neighbours_of_a_diverged_env_are_unchanged(value, asym, E, last, perturb):
     """A joint position of 2^100 / +inf / NaN in one env of a role lane (mid-lane in a full tile, and the last env of
-    the ragged tile) sends that lane down the IEEE path.  Every other env's obs, clipped obs and bf16 obs stay bit for
-    bit those of the run without the plant, noise included; the planted element is the IEEE formula of its value
-    (the noise is below its ulp, or it is not finite), clamped like torch.clamp in the clipped copy."""
+    the ragged tile) sends that lane down the IEEE path.  The planted column carries DR white noise, a per-episode
+    offset, or both.  Every other env's obs, clipped obs and bf16 obs stay bit for bit those of the run without the
+    plant, noise and offset included; the planted element is torch's 2((v + b) - c) / span of its value v and its own
+    offset b (the noise is below its ulp, or it is not finite), clamped like torch.clamp in the clipped copy."""
     from leibnizgym_b200.env import TrifingerEnv
     from leibnizgym_b200.sim import SyntheticSim
     from leibnizgym_b200.synthetic import make_sequence
@@ -473,13 +370,15 @@ def test_noisy_neighbours_of_a_diverged_env_are_unchanged(value, asym, E, last):
     cfg = config(N, asym, 9, "philox", action_noise=False)
     cfg["reward_terms"].pop("keypoint")
     cfg["goal_movement"] = {"rotation": {"activate": False}}
-    cfg["domain_randomization"]["obs_noise_std"] = {"robot_q": 0.01, "robot_u": 0.0, "object_q": 0.0,
-                                                    "object_q_des": 0.0, "command": 0.0}
+    dr = cfg["domain_randomization"]
+    dr["obs_noise_std"] = {"robot_q": 0.01 if perturb != "offset" else 0.0, "robot_u": 0.0, "object_q": 0.0,
+                           "object_q_des": 0.0, "command": 0.0}
+    dr["obs_bias_std"] = {"robot_q": 0.01} if perturb != "noise" else {}
     seq = make_sequence(91, 3, N)
     planted = copy.deepcopy(seq)
     for e in (mid, N - 1):
         planted.dof_state[1:, e, col, 0] = value
-    outs = []
+    outs, biases = [], []
     for sq in (seq, planted):
         env = TrifingerEnv(cfg, device="cuda:0", verbose=False, sim=SyntheticSim(sq.to("cuda:0"), "cuda:0"))
         vec = VecTaskPython(env, rl_device="cuda:0", clip_obs=5.0, clip_actions=1.0, obs_dtype=torch.bfloat16)
@@ -488,19 +387,21 @@ def test_noisy_neighbours_of_a_diverged_env_are_unchanged(value, asym, E, last):
         for t in (1, 2):
             vec.step(seq.action[t].cuda())
             steps.append(tuple(x.clone() for x in (env.obs_buf, env._obs_clipped, env._obs_bf16.view(torch.int16))))
+            biases.append(torch.zeros(2) if env.obs_bias is None else env.obs_bias[[mid, N - 1], col].cpu())
         outs.append(steps)
-    c0, span = np.float32(env._P.scale_centre[col]), np.float32(env._P.scale_span[col])
-    with np.errstate(invalid="ignore", over="ignore"):
-        want = (np.float32(2.0) * (np.float32(value) - c0)) / span
+    assert (perturb == "noise") == all(float(b.abs().sum()) == 0 for b in biases)
+    c0 = torch.tensor(env._P.scale_centre[col], dtype=torch.float32)
+    span = torch.tensor(env._P.scale_span[col], dtype=torch.float32)
     for t, (clean, dirty) in enumerate(zip(*outs)):
+        want = (2.0 * ((torch.full((2,), value) + biases[2 + t]) - c0)) / span
         for k, (a, b) in enumerate(zip(clean, dirty)):
             a, b = a.clone(), b.clone()
             got = _np(b[[mid, N - 1], col].float() if k < 2 else b[[mid, N - 1], col])
             if k < 2:
-                exp = want if k == 0 else np.clip(want, np.float32(-5.0), np.float32(5.0))
-                assert rf_same(got, np.full(2, exp, np.float32)), (t, k, value, got, exp)
+                exp = want if k == 0 else torch.clamp(want, -5.0, 5.0)
+                assert rf_same(got, exp), (t, k, value, perturb, got, exp)
             a[[mid, N - 1], col] = 0
             b[[mid, N - 1], col] = 0
             bad = torch.nonzero(a != b)[:8].tolist()
-            assert not bad, (t, ["obs", "obs_clipped", "obs_bf16"][k], value, (mid, N), bad,
+            assert not bad, (t, ["obs", "obs_clipped", "obs_bf16"][k], value, perturb, (mid, N), bad,
                              [(float(a[i, j]), float(b[i, j])) for i, j in bad])
